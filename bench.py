@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- presentations verified/sec (Issuer::verify, 4 attributes) on N B200s, with the integer-pipe roofline.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--impl native|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--impl native|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
 
 A step = one pass of the hot path over one batch of B = 65,536 README-4 presentations per GPU (BASELINE.json configs[1]).
@@ -619,6 +619,13 @@ def stream_config5(torch, dist, sharded4, rank, world, local, total, stream, cor
     return res
 
 
+def dump_outputs(out_dir, **arrays):
+    """--dump-outputs: each array as out_dir/<name>.npy in float32."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a, np.float32))
+
+
 def run_reference(args, rank):
     """--impl reference: the reference's own CPU schedule of Issuer::verify on the host cores, on the native arm's config.  The Rust
     crate cannot be built in this image (no rustc/cargo, un-vendored deps), so this is the C restatement of its schedule (oracle/c)."""
@@ -641,6 +648,8 @@ def run_reference(args, rank):
         v, rate, wall = cpu_leg(sp, ip, sk, KINDS_README4, items, cores)
         assert not v.any()
         t_total += wall; n_total += B
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, verdicts_reference=v)
     value = n_total / t_total
     line = {"impl": "reference", "metric": "presentations_verified_per_sec", "value": value, "unit": "presentations/s", "n_gpus": args.gpus,
             "steps": args.steps, "warmup": args.warmup, "ms_per_step": 1e3 * t_total / args.steps, "higher_is_better": True, "scaling": "weak",
@@ -664,6 +673,8 @@ def main():
     ap.add_argument("--no-stream", action="store_true", help="skip the config-5 mixed stream")
     ap.add_argument("--stream-items", type=int, default=1 << 22, help="items of the config-5 stream (BASELINE: 2^22)")
     ap.add_argument("--tiled-input", action="store_true", help="tile the 1,024-item CPU-made fixture instead of synthesizing the batch on the device")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the verdicts of the last timed device-resident and end-to-end steps to DIR/<name>.npy "
+                                                          "(float32; the inputs are seeded, so runs with the same arguments compare item for item)")
     args = ap.parse_args()
     rank = int(os.environ.get("RANK", "0")); world = int(os.environ.get("WORLD_SIZE", "1")); local = int(os.environ.get("LOCAL_RANK", "0"))
     if args.impl == "reference":
@@ -759,6 +770,8 @@ def main():
         e2e_s = time.perf_counter() - t0
     gather_ms = 1e3 * sharded.gather_seconds / args.steps
     assert (v == expect).all()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, verdicts_device=verdicts_dev.cpu().numpy(), verdicts_e2e=v)
     # also timed, per rank on its own slice (no gather): the struct-of-arrays entry and the streamed submit / wait form
     host = torch.empty((WORDS, B, 32), dtype=torch.uint8).pin_memory()
     host.numpy()[:] = honest_local.transpose(1, 0, 2)

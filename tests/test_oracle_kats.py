@@ -1,8 +1,6 @@
 """Pins the Python oracle to external known-answer tests (SURVEY 8c): Keccak via hashlib's SHA3,
 merlin's published transcript + STROBE conformance vectors, RFC 9496 constants and generator
-multiples, libsodium 1.0.20 ristretto255 (when loadable), and the reference's own test verdicts."""
-import ctypes
-import glob
+multiples, libsodium 1.0.20 ristretto255 (recorded answers), and the reference's own test verdicts."""
 import hashlib
 import json
 import os
@@ -56,29 +54,25 @@ def test_rfc9496_constants():
 
 def test_rfc9496_appendix_a():
     """RFC 9496 Appendix A in full (tests/golden/rfc9496.json): the 16 generator multiples (A.1), all 29 invalid encodings by
-    group (A.2), hash-to-group (A.3) -- Python oracle, and libsodium 1.0.20 beside it when loadable."""
+    group (A.2), hash-to-group (A.3) -- Python oracle, and libsodium 1.0.20's answers (tests/golden/sodium.json) beside it."""
     g = json.load(open(os.path.join(GOLD, "rfc9496.json")))
-    lib = _sodium()
-    out = ctypes.create_string_buffer(32)
+    sod = _sodium()["rfc9496"]
     assert len(g["multiples"]) == 16
     for k, h in enumerate(g["multiples"]):
         assert (R.BASEPOINT * k).compress().hex() == h
         dec = R.decompress(bytes.fromhex(h))
         assert dec is not None and dec.compress().hex() == h
-        if lib is not None and k:
-            assert lib.crypto_scalarmult_ristretto255(out, k.to_bytes(32, "little"), R.BASEPOINT_COMPRESSED) == 0 and out.raw.hex() == h
+        if k:
+            assert sod["multiples_1_to_15"][k - 1] == h
     assert sum(len(v) for v in g["invalid"].values()) == 29
     for group, encs in g["invalid"].items():
-        for h in encs:
+        for h, valid in zip(encs, sod["invalid_is_valid_point"][group], strict=True):
             assert R.decompress(bytes.fromhex(h)) is None, (group, h)
-            if lib is not None:
-                assert not lib.crypto_core_ristretto255_is_valid_point(bytes.fromhex(h)), (group, h)
-    for e in g["hash_to_group"]:
+            assert not valid, (group, h)
+    for e, sodium_out in zip(g["hash_to_group"], sod["hash_to_group"], strict=True):
         assert hashlib.sha512(e["label"].encode()).hexdigest() == e["input"]
         assert R.from_uniform_bytes(bytes.fromhex(e["input"])).compress().hex() == e["output"]
-        if lib is not None:
-            lib.crypto_core_ristretto255_from_hash(out, bytes.fromhex(e["input"]))
-            assert out.raw.hex() == e["output"]
+        assert sodium_out == e["output"]
 
 
 def test_transcript_regression_vector_v1():
@@ -91,40 +85,30 @@ def test_transcript_regression_vector_v1():
 
 
 def _sodium():
-    for path in glob.glob("/opt/prime-rl/.venv/lib/python3*/site-packages/pyzmq.libs/libsodium*.so*"):
-        try:
-            lib = ctypes.CDLL(path)
-            lib.crypto_core_ristretto255_from_hash
-            lib.sodium_init()
-            return lib
-        except (OSError, AttributeError):
-            continue
-    return None
+    """libsodium's outputs on the inputs of these tests, recorded by tests/golden/make_sodium.py."""
+    return json.load(open(os.path.join(GOLD, "sodium.json")))
 
 
 def test_against_libsodium():
-    lib = _sodium()
-    if lib is None:
-        pytest.skip("libsodium with ristretto255 not loadable")
+    rounds = _sodium()["rounds"]
     rng = A.ShakeRng(b"sodium")
-    out = ctypes.create_string_buffer(32)
-    for _ in range(60):
+    assert len(rounds) == 60
+    for r in rounds:
         b = rng.fill(32)
-        assert (R.decompress(b) is not None) == bool(lib.crypto_core_ristretto255_is_valid_point(b))
+        assert b.hex() == r["b"]
+        assert (R.decompress(b) is not None) == r["b_valid"]
         h = rng.fill(64)
-        lib.crypto_core_ristretto255_from_hash(out, h)
+        assert h.hex() == r["h"]
         P = R.from_uniform_bytes(h)
-        assert P.compress() == out.raw
-        enc = out.raw
+        assert P.compress().hex() == r["from_hash"]
         s = rng.scalar()
-        assert lib.crypto_scalarmult_ristretto255(out, R.sc_to_bytes(s), enc) == 0
-        assert (P * s).compress() == out.raw
+        assert R.sc_to_bytes(s).hex() == r["s"]
+        assert (P * s).compress().hex() == r["scalarmult"]
         h2 = rng.fill(64)
+        assert h2.hex() == r["h2"]
         Q = R.from_uniform_bytes(h2)
-        lib.crypto_core_ristretto255_sub(out, enc, Q.compress())
-        assert (P - Q).compress() == out.raw
-        lib.crypto_core_ristretto255_scalar_reduce(out, h)
-        assert R.sc_to_bytes(R.sc_from_wide(h)) == out.raw
+        assert (P - Q).compress().hex() == r["sub"]
+        assert R.sc_to_bytes(R.sc_from_wide(h)).hex() == r["scalar_reduce"]
 
 
 def test_golden_prims():

@@ -1,9 +1,9 @@
 import os, sys, time
 import numpy as np
-sys.path.insert(0, "/root/repo")
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT)
 import torch
 from aeonflux_b200 import Issuer, PresentationBatch, compact_to_batchable
-ROOT = "/root/repo"
 blob = open(os.path.join(ROOT, "bench_data", "issuer16.bin"), "rb").read()
 pres = np.fromfile(os.path.join(ROOT, "bench_data", "s16_256.bin"), np.uint8).reshape(-1, 143, 32)
 sp, ip, sk = blob[:1316], blob[1316:1380], blob[1380:]
