@@ -405,18 +405,25 @@ static void allow_large_smem(const void* kernel, int which) {
     }
 }
 
-// One launch for the aMAC ladder (if `amac`) plus the MSMs of one scratch-size group.
-// The last n_dep_jobs entries of d_idx are the MSMs that wait on the aMAC flags.
-static u32 be_launch_ladders(const Workspace& ws, const AmacDesc* amac, u32 amac_nps, const MsmDesc* d_msms, const u32* d_idx, u32 nidx, u32 n_dep_jobs,
-                             u32 max_terms, u32 amac_terms, int dep_msm, u32* flags, u32 epoch, u32 flag_tpb, u32* ticket, be_stream s) {
-    u32 terms = max_terms > amac_nps ? max_terms : amac_nps;
-    // largest CTA (<= TPB_MSM threads) whose digit scratch fits in shared memory
+// Launch geometry of a ladder kernel whose CTAs hold `terms` terms of digit scratch: the largest CTA (<= TPB_MSM threads) whose
+// scratch fits LADDER_SMEM_BUDGET, and that scratch in bytes.
+struct LadderGeometry { u32 tpb; size_t smem; };
+static LadderGeometry ladder_geometry(u32 terms) {
     u32 tpb = TPB_MSM;
     size_t smem = 0;
     for (;; tpb /= 2) {
         smem = (size_t)terms * 8 * tpb * 4;
         if (smem <= LADDER_SMEM_BUDGET || tpb <= 32) break;
     }
+    return {tpb, smem};
+}
+
+// One launch for the aMAC ladder (if `amac`) plus the MSMs of one scratch-size group.
+// The last n_dep_jobs entries of d_idx are the MSMs that wait on the aMAC flags.
+static u32 be_launch_ladders(const Workspace& ws, const AmacDesc* amac, u32 amac_nps, const MsmDesc* d_msms, const u32* d_idx, u32 nidx, u32 n_dep_jobs,
+                             u32 max_terms, u32 amac_terms, int dep_msm, u32* flags, u32 epoch, u32 flag_tpb, u32* ticket, be_stream s) {
+    u32 terms = max_terms > amac_nps ? max_terms : amac_nps;
+    const auto [tpb, smem] = ladder_geometry(terms);
     allow_large_smem((const void*)k_ladders, 0);
     const u32 nx = (ws.count + tpb - 1) / tpb;
     const u32 n_dep = n_dep_jobs < nidx ? n_dep_jobs : nidx, n_ind = nidx - n_dep;
@@ -452,12 +459,7 @@ static void be_launch_ladders_parts(const Workspace& ws, const AmacDesc* amac, c
                                     const MsmDesc* d_msms, const u32* d_idx, u32 nidx, u32 max_terms, be_stream s) {
     u32 terms = max_terms > part_terms ? max_terms : part_terms;
     if (terms < 1) terms = 1;
-    u32 tpb = TPB_MSM;
-    size_t smem = 0;
-    for (;; tpb /= 2) {
-        smem = (size_t)terms * 8 * tpb * 4;
-        if (smem <= LADDER_SMEM_BUDGET || tpb <= 32) break;
-    }
+    const auto [tpb, smem] = ladder_geometry(terms);
     allow_large_smem((const void*)k_ladders_parts, 2);
     PartsArgs a;
     a.msms = d_msms; a.group_idx = d_idx; a.scratch_terms = terms; a.amac = amac; a.parts_out = parts_out; a.n_parts = n_parts;
@@ -469,12 +471,7 @@ static void be_launch_amac_combine(const Workspace& ws, const AmacDesc* amac, co
     k_amac_combine<<<grid_for(ws.count, 128, 1), 128, 0, s>>>(ws, amac, parts_out, n_parts);
 }
 static void be_launch_msm_ct(const Workspace& ws, const MsmDesc* d_msms, const u32* d_idx, u32 nidx, u32 max_terms, be_stream s) {
-    u32 tpb = TPB_MSM;
-    size_t smem = 0;
-    for (;; tpb /= 2) {
-        smem = (size_t)max_terms * 8 * tpb * 4;
-        if (smem <= LADDER_SMEM_BUDGET || tpb <= 32) break;
-    }
+    const auto [tpb, smem] = ladder_geometry(max_terms);
     allow_large_smem((const void*)k_msm_ct, 1);
     k_msm_ct<<<grid_for(ws.count, tpb, nidx), tpb, smem, s>>>(ws, d_msms, d_idx);
 }

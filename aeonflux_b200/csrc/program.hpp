@@ -455,6 +455,7 @@ inline ShapeProgram compile_presentation(const IssuerConsts& ic, u32 n, const ui
 // kinds: 0 = scalar attribute (M_i = m_i * G_m[i]), 2 = point attribute.  Fields: attr[n], t, U, V, challenge, responses[n+5].
 // batchable = the same statement verified from a BatchableProof (the commented-out BatchVerifier of issuance.rs:21-22): the
 // challenge word is replaced by the three blinding commitments (constraint order C_W, I, V), i.e. 2n + 11 fields.
+inline size_t issuance_num_fields(u32 n) { return 2 * (size_t)n + 9; }
 inline size_t issuance_batchable_num_fields(u32 n) { return 2 * (size_t)n + 11; }
 inline ShapeProgram compile_issuance_verify(const IssuerConsts& ic, u32 n, const uint8_t* kinds, bool batchable = false) {
     if (n != ic.n || n == 0 || n > MAX_ATTRS) throw std::invalid_argument("attribute count does not match the issuer's");
@@ -462,7 +463,7 @@ inline ShapeProgram compile_issuance_verify(const IssuerConsts& ic, u32 n, const
     ShapeProgram P;
     P.batchable = batchable;
     const u32 F_ATTR = 0, F_T = n, F_U = n + 1, F_V = n + 2, F_CHAL = n + 3, F_RESP = n + 4 + (batchable ? 2 : 0);
-    P.n_fields = 2 * n + 9 + (batchable ? 2 : 0);
+    P.n_fields = (u32)(batchable ? issuance_batchable_num_fields(n) : issuance_num_fields(n));
     // responses: w, w', x_0, x_1, y[n], 1  (issuance.rs:146-159)
     const u32 R_w = F_RESP, R_wp = F_RESP + 1, R_x0 = F_RESP + 2, R_x1 = F_RESP + 3, R_y = F_RESP + 4, R_one = F_RESP + 4 + n;
     for (u32 i = 0; i < n; i++) if (kinds[i] == 0) P.scalar_fields.push_back((u16)(F_ATTR + i));

@@ -351,12 +351,9 @@ const char* afx_version(void);
 
 /* Environment (read by the library, all optional):
  *   AFX_CTAB16_BUDGET_MB   device-memory budget for the radix-2^16 constant tables of one issuer (default 200; 0 = radix 4096 only)
- *   AFX_COPY_PARTS         1..8: contiguous item ranges a one-pass item-major host call copies its batch in, the early per-item
- *                          stages of range k running under the copy of range k + 1 (default 4)
  *   AFX_AMAC_SPLIT         0: never cut the aMAC ladder of a small pass into parts; g > 0: g terms per part for every pass of at most
  *                          32,768 items (default: passes of at most 8,192 items, 2 or 4 terms per part -- DESIGN.md section 5)
  *   AFX_RLC_LEAF           smallest range the bisection of a failing random-linear-combination chunk descends to (default 1024)
- *   AFX_STREAM_RAMP_DIV    afx_stream_*: the first bucket after a flush is 1/div of a full one, later ones double (default 8; 1 = no ramp)
  *   AFX_STREAM_TRACE       non-empty: afx_stream_* logs every bucket submission and retirement with timestamps to stderr */
 
 #ifdef __cplusplus
