@@ -36,7 +36,9 @@ class Binding:
                "afx_verify_presentations_wire_submit", "afx_verify_issuances_wire_submit", "afx_stream_create", "afx_stream_destroy",
                "afx_stream_add_shape", "afx_stream_push", "afx_stream_flush", "afx_stream_buckets_submitted", "afx_stream_times",
                "afx_issue_wire", "afx_show_wire", "afx_presentation_linked_num_commitments", "afx_verify_presentations_linked",
-               "afx_verify_presentations_linked_wire", "afx_show_linked", "afx_show_linked_wire", "afx_issuance_batchable_num_fields", "afx_verify_issuances_batchable", "afx_verify_issuances_batchable_rlc", "afx_get_rlc_stats"]
+               "afx_verify_presentations_linked_wire", "afx_show_linked", "afx_show_linked_wire", "afx_issuance_batchable_num_fields", "afx_verify_issuances_batchable", "afx_verify_issuances_batchable_rlc", "afx_get_rlc_stats",
+               "afx_encode_plaintexts", "afx_encrypt", "afx_decrypt", "afx_encode_plaintexts_device", "afx_encrypt_device",
+               "afx_decrypt_device"]
 
     def __init__(self, cdll):
         L = self.L = cdll
@@ -105,6 +107,18 @@ class Binding:
         for f in ("afx_issue_wire", "afx_show_wire", "afx_show_linked_wire"):
             getattr(L, f).restype = ctypes.c_int
             getattr(L, f).argtypes = [vp, ctypes.c_uint16, ctypes.c_char_p, sz, vp, vp, vp]
+        L.afx_encode_plaintexts.restype = ctypes.c_int
+        L.afx_encode_plaintexts.argtypes = [vp, sz, vp, vp, vp]
+        L.afx_encrypt.restype = ctypes.c_int
+        L.afx_encrypt.argtypes = [vp, vp, sz, vp, vp, vp]
+        L.afx_decrypt.restype = ctypes.c_int
+        L.afx_decrypt.argtypes = [vp, vp, sz, vp, vp, vp, vp]
+        L.afx_encode_plaintexts_device.restype = ctypes.c_int
+        L.afx_encode_plaintexts_device.argtypes = [vp, sz, vp, vp, vp, vp]
+        L.afx_encrypt_device.restype = ctypes.c_int
+        L.afx_encrypt_device.argtypes = [vp, vp, sz, vp, vp, vp, vp]
+        L.afx_decrypt_device.restype = ctypes.c_int
+        L.afx_decrypt_device.argtypes = [vp, vp, sz, vp, vp, vp, vp, vp]
         L.afx_selftest_primitive.restype = ctypes.c_int
         L.afx_selftest_primitive.argtypes = [vp, ctypes.c_int, vp, sz, vp, vp]
         L.afx_launch_count.restype = ctypes.c_uint64

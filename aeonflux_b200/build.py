@@ -5,7 +5,7 @@ import subprocess
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 SO = os.path.join(CSRC, "libaeonflux_b200.so")
-SOURCES = ["afx_b200.cu", "api_impl.inc", "engine.cuh", "fe.cuh", "ge.cuh", "sc.cuh", "keccak.cuh", "program.hpp"]
+SOURCES = ["afx_b200.cu", "api_impl.inc", "engine.cuh", "fe.cuh", "ge.cuh", "sc.cuh", "keccak.cuh", "sha512.cuh", "program.hpp"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17", "-Xcompiler", "-fPIC,-fvisibility=hidden", "-shared"]
 
 

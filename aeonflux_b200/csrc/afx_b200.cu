@@ -298,6 +298,16 @@ __global__ void __launch_bounds__(128) k_primitive(u32 op, const u32* in, u32* o
     u32 item = blockIdx.x * blockDim.x + threadIdx.x;
     if (item < count) primitive_job(op, in, out, flags, item);
 }
+// symmetric encryption of attributes: one thread per item (engine.cuh:encode_job / decrypt_job)
+__global__ void __launch_bounds__(128) k_encode(const uint8_t* data, u32* pt, uint8_t* status, u32 count, u32 item_major) {
+    u32 item = blockIdx.x * blockDim.x + threadIdx.x;
+    if (item < count) encode_job(data, pt, status, count, item_major, item);
+}
+__global__ void __launch_bounds__(128) k_decrypt(const u32* ct, const u32* kp, u32* tabs, uint8_t* data, u32* pt, uint8_t* status, u32 count,
+                                                 u32 item_major) {
+    u32 item = blockIdx.x * blockDim.x + threadIdx.x;
+    if (item < count) decrypt_job(ct, kp, tabs, data, pt, status, count, item_major, item);
+}
 __global__ void k_secret_setup(const u32* secsc, u32 nsec, u32* secdig, const u32* Wenc, u32* W_pniels, u32* bad) {
     u32 t = blockIdx.x * blockDim.x + threadIdx.x;
     if (t < nsec) {
@@ -532,6 +542,12 @@ static void be_launch_primitive(u32 op, const u32* in, u32* out, u32* flags, u32
 }
 static void be_launch_secret_setup(const u32* d_secsc, u32 nsec, u32* d_secdig, const u32* d_Wenc, u32* d_W, u32* d_bad, be_stream s) {
     k_secret_setup<<<1, 64, 0, s>>>(d_secsc, nsec, d_secdig, d_Wenc, d_W, d_bad);
+}
+static void be_launch_encode(const uint8_t* data, u32* pt, uint8_t* status, u32 count, bool item_major, be_stream s) {
+    k_encode<<<grid_for(count, 128, 1), 128, 0, s>>>(data, pt, status, count, item_major);
+}
+static void be_launch_decrypt(const u32* ct, const u32* kp, u32* tabs, uint8_t* data, u32* pt, uint8_t* status, u32 count, bool item_major, be_stream s) {
+    k_decrypt<<<grid_for(count, 128, 1), 128, 0, s>>>(ct, kp, tabs, data, pt, status, count, item_major);
 }
 
 #include "api_impl.inc"

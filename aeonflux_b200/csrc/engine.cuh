@@ -14,11 +14,13 @@
 //   transcript one thread per (item, proof): Merlin/STROBE/Keccak-f[1600] over the compiled block template, 64-byte
 //              challenge squeeze, reduction mod l, compare with the claimed challenge
 //   verdict    status word -> 0 (Ok) / 1 (VerificationFailure)
+// Symmetric encryption of attributes (encoding.rs, symmetric.rs) has its own per-item bodies at the end of this file.
 #pragma once
 #include "fe.cuh"
 #include "ge.cuh"
 #include "keccak.cuh"
 #include "sc.cuh"
+#include "sha512.cuh"
 
 namespace afx {
 
@@ -1045,6 +1047,109 @@ AFX_HD void comb_entry_job(const u32* enc /*8 words*/, u32 i, u32 e, u32* out /*
     store_fe(out, fe_add(y, x));
     store_fe(out + 8, fe_sub(y, x));
     store_fe(out + 16, fe_mul(fe_mul(x, y), FE_D2()));
+}
+
+// ---- symmetric encryption of attributes (encoding.rs:56-82, symmetric.rs:89-96,135-143,252-261,273-289) --------------------------
+// Keypair::encrypt is a program of the prover stages (program.hpp:compile_encrypt); encoding and decryption are one thread per item.
+// Word w of the nw words of an item: item-major [count][nw][8] (the host calls) or struct-of-arrays [nw][count][8] (the *_device calls).
+AFX_HD size_t sym_word(u32 count, u32 nw, u32 item_major, u32 w, u32 item) {
+    return (item_major ? (size_t)item * nw + w : (size_t)w * count + item) * 8;
+}
+
+// Plaintext::from(&[u8; 30]): M1 = the first candidate 2i || data || j (j = 0..63, i = 0..127) that decompresses, h = SHA-512(data),
+// M2 = from_uniform_bytes(h), m3 = h mod l.  Variable time in the number of candidates, as the reference's loop.  status 1 (all-zero
+// words) when no candidate decodes, where the reference panics.
+AFX_HD void encode_job(const uint8_t* data /*[count][30]*/, u32* pt, uint8_t* status, u32 count, u32 item_major, u32 item) {
+    enc32 base;      // 0 || data || 0
+    for (int w = 0; w < 8; w++) {
+        u32 v = 0;
+        for (int b = 0; b < 4; b++) { const int k = 4 * w + b - 1; if (k >= 0 && k < 30) v |= (u32)data[(size_t)item * 30 + k] << (8 * b); }
+        base.w[w] = v;
+    }
+    u32 enc[8], found = 0;
+    ge p;
+    for (u32 k = 0; k < 64 * 128; k++) {
+        for (int w = 0; w < 8; w++) enc[w] = base.w[w];
+        enc[0] |= 2u * (k & 127u); enc[7] |= (k >> 7) << 24;
+        if (ge_decompress(p, enc)) { found = 1; break; }
+    }
+    const digest64 h = sha512_30(base);
+    u32 m2[8];
+    ge_compress(m2, ge_from_uniform(h.w));
+    const sc m3 = sc_reduce512(h.w);
+    const u32 m = 0u - found;
+    u32 m3w[8];
+    for (int i = 0; i < 8; i++) { enc[i] &= m; m2[i] &= m; m3w[i] = m3.v[i] & m; }
+    store8(pt + sym_word(count, 3, item_major, 0, item), enc);
+    store8(pt + sym_word(count, 3, item_major, 1, item), m2);
+    store8(pt + sym_word(count, 3, item_major, 2, item), m3w);
+    status[item] = (uint8_t)(found ^ 1u);
+}
+
+// k * P for a secret k over P's [1P..8P] table (warp-transposed, scan-and-mask reads): 64 signed radix-16 digits, every digit added,
+// so neither the instruction stream nor the address stream depends on k.  The digits stay in registers.
+AFX_NI ge ct_ladder(const u32* tab, sc k) {
+    u32 rec[8];
+    sc_recode16(rec, k);
+    gc acc = gc_identity();
+#if defined(__CUDA_ARCH__)
+#pragma unroll 1
+#endif
+    for (int i = 63; i >= 0; i--) {
+        if (i != 63) gc_dbl4(acc);
+        u32 word = rec[0];
+        for (int j = 1; j < 8; j++) word = (i >> 3) == j ? rec[j] : word;     // public index: selects, not a local-memory array
+        pniels e = pniels_scan_select_t(tab, ((int)(word << (28 - 4 * (i & 7)))) >> 28);
+        GE_LADDER_ADD(acc, e);
+    }
+    return gc_to_ge(acc);
+}
+
+// a0 + a1*m3 (a subroutine: its unrolled limb products would otherwise share the registers of decrypt_job's live points)
+AFX_NI sc decrypt_u(const u32* kp, sc m3) { return sc_muladd(load_sc(kp + 16), m3, load_sc(kp + 8)); }
+
+// Keypair::decrypt: M1' = E2 - a*E1, data' = compress(M1')[1..31], h = SHA-512(data'), M2' = from_uniform_bytes(h), m3' = h mod l;
+// accept iff (a0 + a1*m3')*M2' == E1.  kp = a, a0, a1 (canonical).  tabs: warp-transposed ladder tables, one per item, used by both
+// ladders.  Outputs (data [count][30], the Plaintext words when pt != null) are all-zero and status is 1 when E1 or E2 does not
+// decode or the check fails (CredentialError::UndecryptableAttribute).
+AFX_HD void decrypt_job(const u32* ct, const u32* kp, u32* tabs, uint8_t* data, u32* pt, uint8_t* status, u32 count, u32 item_major, u32 item) {
+    // The outputs are written as soon as they exist and cleared if the check fails, so that nothing but `ok` and the pointers stays
+    // live across the ladders (the calls would otherwise spill it).
+    u32* tab = tabs + (size_t)(item / 32) * ATAB_BLOCK_WORDS + (item % 32) * 4;
+    u32 w[8];
+    load8(w, ct + sym_word(count, 2, item_major, 0, item));
+    ge p;
+    u32 ok = ge_decompress(p, w);
+    store_table8(nullptr, p, tab);
+    const ge aE1 = ct_ladder(tab, load_sc(kp));
+    load8(w, ct + sym_word(count, 2, item_major, 1, item));
+    ok &= ge_decompress(p, w);
+    const enc32 m1 = ge_compress_v(ge_sub(p, aE1));
+    uint8_t* d = data + (size_t)item * 30;
+    for (int k = 0; k < 30; k++) d[k] = (uint8_t)(m1.w[(k + 1) >> 2] >> (8 * ((k + 1) & 3)));
+    if (pt) store8(pt + sym_word(count, 3, item_major, 0, item), m1.w);
+    const digest64 h = sha512_30(m1);
+    p = ge_from_uniform(h.w);
+    const sc m3 = sc_reduce512(h.w);
+    if (pt) {
+        ge_compress(w, p);
+        store8(pt + sym_word(count, 3, item_major, 1, item), w);
+        store8(pt + sym_word(count, 3, item_major, 2, item), m3.v);
+    }
+    store_table8(nullptr, p, tab);
+    const ge E1 = ct_ladder(tab, decrypt_u(kp, m3));
+    u32 e1[8];
+    ge_compress(w, E1);
+    load8(e1, ct + sym_word(count, 2, item_major, 0, item));
+    u32 x = 0;
+    for (int i = 0; i < 8; i++) x |= w[i] ^ e1[i];
+    ok &= (u32)(x == 0);
+    if (!ok) {     // the verdict is public
+        for (int k = 0; k < 30; k++) d[k] = 0;
+        for (int i = 0; i < 8; i++) w[i] = 0;
+        if (pt) for (u32 k = 0; k < 3; k++) store8(pt + sym_word(count, 3, item_major, k, item), w);
+    }
+    status[item] = (uint8_t)(ok ^ 1u);
 }
 
 }  // namespace afx

@@ -804,4 +804,27 @@ inline ShapeProgram compile_show(const IssuerConsts& ic, u32 n, const uint8_t* k
     return P;
 }
 
+// Keypair::encrypt (symmetric.rs:252-261) as a program: the two ladders of show's proof of encryption (compile_show),
+//     E1 = (a0 + a1*m3)*M2,   E2 = (a*(a0 + a1*m3))*M2 + M1.
+// Fields: the Plaintext M1, M2, m3.  The keypair a, a0, a1 is the call's: the pass puts it in the secret rows (ws.secsc) 0, 1, 2.
+// Output words: E1, E2.  Every scalar is secret (constant-schedule ladders); the derived scalars are wiped after each pass.
+inline ShapeProgram compile_encrypt() {
+    ShapeProgram P; P.is_issue = true;
+    const u32 F_M1 = 0, F_M2 = 1, F_M3 = 2;
+    P.n_fields = 3;
+    P.scalar_fields.push_back((u16)F_M3);
+    auto dv = [&](u32 op, u32 a, u32 b, u32 c = 0) { DeriveOp d; d.op = (u16)op; d.a = (u16)a; d.b = (u16)b; d.c = (u16)c; P.derived.push_back(d); return sref_derived((u32)P.derived.size() - 1); };
+    const u32 D_u = dv(DV_MULADD, sref_secret(1), sref_secret(2), F_M3);      // a0 + a1*m3
+    const u32 D_au = dv(DV_MUL, sref_secret(0), D_u);
+    PointJob j; j.field_b = -1; j.op = PJ_COPY; j.table_slot = -1; j.comp_slot = -1; j.compneg_slot = -1;
+    j.field_a = (int16_t)F_M1; j.atab_slot = -1; j.ext_slot = 0; P.point_jobs.push_back(j);
+    j.field_a = (int16_t)F_M2; j.atab_slot = 0; j.ext_slot = -1; P.point_jobs.push_back(j);
+    P.n_tables = 0; P.n_atabs = 1; P.n_ext = 1; P.n_comp = 0;
+    { MsmBuilder m(0); m.var(0, sc_field(D_u)); P.msms.push_back(m.d); }
+    { MsmBuilder m(1); m.var(0, sc_field(D_au)); m.add_ext(0); P.msms.push_back(m.d); }
+    P.n_msm = 2; P.n_proofs = 0;
+    for (u32 k = 0; k < 2; k++) { OutWord o; o.kind = OW_COMMIT; o.a = (u16)k; o.b = o.c = 0; P.out_words.push_back(o); }
+    return P;
+}
+
 }  // namespace afx

@@ -384,6 +384,96 @@ class Issuer:
     def verify_issuance_batch_device(self, kinds, count, fields_dev_ptr, verdicts_dev_ptr, stream=0):
         self._b.check(self._b.L.afx_verify_issuances_device(self._h, len(kinds), bytes(kinds), count, fields_dev_ptr, verdicts_dev_ptr, stream))
 
+    # -- symmetric encryption of attributes (encoding.rs, symmetric.rs); the calls need no issuer secret
+    @staticmethod
+    def _array(name, a, shape):
+        if not isinstance(a, np.ndarray) or a.dtype != np.uint8 or a.shape != shape or not a.flags.c_contiguous:
+            raise ValueError("%s must be a contiguous uint8 %s array" % (name, "[" + "][".join(str(d) for d in shape) + "]"))
+        return a
+
+    @staticmethod
+    def _keypair(keypair):
+        """keypair: a || a0 || a1 (96 bytes), or the 128-byte keypair show takes (a, a0, a1, pk)."""
+        kp = bytes(keypair)
+        if len(kp) not in (96, 128):
+            raise ValueError("keypair must be a || a0 || a1 (96 bytes) or a || a0 || a1 || pk (128 bytes)")
+        return ctypes.create_string_buffer(kp[:96], 96)
+
+    def encode_plaintexts(self, data, out=None):
+        """Plaintext::from(&[u8; 30]) for every row of data (uint8 [count][30]) -> (plaintexts uint8 [count][3][32]: M1, M2, m3 --
+        the words of a hidden plaintext attribute in show's input, status).  status 1 (all-zero words): no candidate encoding of
+        the 8,192 decodes (the reference panics there)."""
+        data = np.asarray(data, dtype=np.uint8)
+        if data.ndim != 2 or data.shape[1] != 30:
+            raise ValueError("data must be [count][30] bytes")
+        data = np.ascontiguousarray(data)
+        count = data.shape[0]
+        out = np.zeros((count, 3, 32), np.uint8) if out is None else self._array("out", out, (count, 3, 32))
+        status = np.zeros(count, np.uint8)
+        self._b.check(self._b.L.afx_encode_plaintexts(self._h, count, data.ctypes.data, out.ctypes.data, status.ctypes.data))
+        return out, status
+
+    def encrypt(self, keypair, plaintexts, out=None):
+        """Keypair::encrypt (symmetric.rs:252-261) of every Plaintext (uint8 [count][3][32]: M1, M2, m3) -> (ciphertexts uint8
+        [count][2][32]: E1, E2, status).  status 1 (all-zero words): M1 or M2 does not decode, or m3 is not canonical."""
+        kp = self._keypair(keypair)
+        plaintexts = np.asarray(plaintexts, dtype=np.uint8)
+        if plaintexts.ndim != 3 or plaintexts.shape[1:] != (3, 32):
+            raise ValueError("plaintexts must be [count][3][32] bytes")
+        plaintexts = np.ascontiguousarray(plaintexts)
+        count = plaintexts.shape[0]
+        out = np.zeros((count, 2, 32), np.uint8) if out is None else self._array("out", out, (count, 2, 32))
+        status = np.zeros(count, np.uint8)
+        try:
+            self._b.check(self._b.L.afx_encrypt(self._h, ctypes.addressof(kp), count, plaintexts.ctypes.data, out.ctypes.data, status.ctypes.data))
+        finally:
+            ctypes.memset(kp, 0, 96)
+        return out, status
+
+    def decrypt(self, keypair, ciphertexts, plaintexts=False, out=None):
+        """Keypair::decrypt (symmetric.rs:273-289) of every ciphertext (uint8 [count][2][32]: E1, E2) -> (data uint8 [count][30],
+        status), or (data, plaintexts uint8 [count][3][32], status) with plaintexts=True.  status 1 (all-zero output):
+        CredentialError::UndecryptableAttribute, or E1 / E2 does not decode."""
+        kp = self._keypair(keypair)
+        ciphertexts = np.asarray(ciphertexts, dtype=np.uint8)
+        if ciphertexts.ndim != 3 or ciphertexts.shape[1:] != (2, 32):
+            raise ValueError("ciphertexts must be [count][2][32] bytes")
+        ciphertexts = np.ascontiguousarray(ciphertexts)
+        count = ciphertexts.shape[0]
+        data = np.zeros((count, 30), np.uint8) if out is None else self._array("out", out, (count, 30))
+        pts = np.zeros((count, 3, 32), np.uint8) if plaintexts else None
+        status = np.zeros(count, np.uint8)
+        try:
+            self._b.check(self._b.L.afx_decrypt(self._h, ctypes.addressof(kp), count, ciphertexts.ctypes.data, data.ctypes.data,
+                                                pts.ctypes.data if plaintexts else None, status.ctypes.data))
+        finally:
+            ctypes.memset(kp, 0, 96)
+        return (data, pts, status) if plaintexts else (data, status)
+
+    def encode_plaintexts_device(self, count, data_dev_ptr, plaintexts_dev_ptr, status_dev_ptr, stream=0):
+        """Enqueue encode_plaintexts on device memory: data [count][30] -> plaintexts [3][count][32] (the rows show_batch_device takes
+        for a hidden plaintext), status [count]; count <= max_batch, no synchronisation."""
+        self._b.check(self._b.L.afx_encode_plaintexts_device(self._h, count, data_dev_ptr, plaintexts_dev_ptr, status_dev_ptr, stream))
+
+    def encrypt_device(self, keypair, count, plaintexts_dev_ptr, ciphertexts_dev_ptr, status_dev_ptr, stream=0):
+        """Enqueue encrypt on device memory: plaintexts [3][count][32] -> ciphertexts [2][count][32], status [count]."""
+        kp = self._keypair(keypair)
+        try:
+            self._b.check(self._b.L.afx_encrypt_device(self._h, ctypes.addressof(kp), count, plaintexts_dev_ptr, ciphertexts_dev_ptr,
+                                                       status_dev_ptr, stream))
+        finally:
+            ctypes.memset(kp, 0, 96)
+
+    def decrypt_device(self, keypair, count, ciphertexts_dev_ptr, data_dev_ptr, status_dev_ptr, plaintexts_dev_ptr=None, stream=0):
+        """Enqueue decrypt on device memory: ciphertexts [2][count][32] -> data [count][30], optional plaintexts [3][count][32],
+        status [count]."""
+        kp = self._keypair(keypair)
+        try:
+            self._b.check(self._b.L.afx_decrypt_device(self._h, ctypes.addressof(kp), count, ciphertexts_dev_ptr, data_dev_ptr,
+                                                       plaintexts_dev_ptr, status_dev_ptr, stream))
+        finally:
+            ctypes.memset(kp, 0, 96)
+
     PRIMITIVES = {"decompress_compress": (0, 32), "from_uniform": (1, 64), "scalarmult": (2, 64), "wide_reduce": (3, 64), "sc_muladd": (4, 96),
                   "fe_mul": (5, 64), "fe_sq": (6, 64), "fe_add": (7, 64), "fe_sub": (8, 64), "fe_chain": (9, 64), "ladder_scalarmult": (10, 64), "recode4096": (11, 32)}
 

@@ -243,6 +243,37 @@ int afx_show_device(afx_ctx* ctx, uint16_t n_attrs, const uint8_t* kinds, size_t
 int afx_show_wire(afx_ctx* ctx, uint16_t n_attrs, const uint8_t* kinds, size_t count, const uint8_t* inputs, uint8_t* presentations,
                   uint8_t* status);
 
+/* Symmetric encryption of attributes: Plaintext::from(&[u8; 30]) (src/symmetric.rs:135-143 -> src/encoding.rs:56-70),
+ * Keypair::encrypt (src/symmetric.rs:252-261) and Keypair::decrypt (src/symmetric.rs:273-289), in batch form.  User-side and
+ * key-holder operations: they need no issuer secret (a context created with secret = NULL suffices) and do not use the system
+ * parameters.  Calls lock the context like every other call.
+ *   data       = [count][30] bytes, the attribute's plaintext bytes
+ *   plaintext  = the words M1, M2, m3 (src/symmetric.rs:89-96): exactly the three words a kind-3 attribute takes in afx_show's input
+ *   ciphertext = the words E1, E2 (src/symmetric.rs:252-261): words 8 and 9 of a presentation's 14-word proof-of-encryption block
+ *   keypair    = a || a0 || a1, 96 bytes of canonical scalars (src/symmetric.rs:74-79): the first 96 bytes of the 128-byte keypair
+ *                afx_show takes.  A scalar >= l is AFX_ERR_ENCODING, and nothing is written.
+ * Host calls are item-major (plaintexts [count][3][32], ciphertexts [count][2][32]) and run in passes of max_batch items.  The
+ * *_device calls take struct-of-arrays device memory (plaintexts [3][count][32], ciphertexts [2][count][32]; data [count][30]),
+ * count <= max_batch, and are enqueued on `stream` (a cudaStream_t; NULL = default stream) without synchronizing, so the rows
+ * afx_encode_plaintexts_device writes can be handed to afx_show_device as they are.
+ * status: 0 = Ok, 1 = the item's output words are all zero and:
+ *   encode:  none of the 8,192 candidate encodings of M1 decodes (the reference panics; no such input is known);
+ *   encrypt: M1 or M2 does not decode, or m3 is not canonical;
+ *   decrypt: E1 or E2 does not decode, or (a0 + a1*m3')*M2' != E1 (CredentialError::UndecryptableAttribute, src/errors.rs).
+ * Timing: encrypt and decrypt run constant-schedule ladders with constant-address table scans (the keypair, m3 and the plaintext are
+ * secrets); the device copy of the keypair, the scalars derived from it and decrypt's ladder tables are zeroed on the stream at the
+ * end of every pass.  Encode runs in variable time, in the number of candidates tried, as the reference's loop does. */
+int afx_encode_plaintexts(afx_ctx* ctx, size_t count, const uint8_t* data, uint8_t* plaintexts, uint8_t* status);
+int afx_encrypt(afx_ctx* ctx, const uint8_t keypair[96], size_t count, const uint8_t* plaintexts, uint8_t* ciphertexts, uint8_t* status);
+/* plaintexts (nullable): the Plaintext (M1', M2', m3') the reference returns. */
+int afx_decrypt(afx_ctx* ctx, const uint8_t keypair[96], size_t count, const uint8_t* ciphertexts, uint8_t* data, uint8_t* plaintexts,
+                uint8_t* status);
+int afx_encode_plaintexts_device(afx_ctx* ctx, size_t count, const void* data_dev, void* plaintexts_dev, void* status_dev, void* stream);
+int afx_encrypt_device(afx_ctx* ctx, const uint8_t keypair[96], size_t count, const void* plaintexts_dev, void* ciphertexts_dev,
+                       void* status_dev, void* stream);
+int afx_decrypt_device(afx_ctx* ctx, const uint8_t keypair[96], size_t count, const void* ciphertexts_dev, void* data_dev,
+                       void* plaintexts_dev, void* status_dev, void* stream);
+
 /* Linked presentations (opt-in; NOT the reference's protocol but the fix its authors left as a TODO: README.md:119-122,
  * src/nizk/presentation.rs:292 "don't we also need DLEQ between the plaintext here and that in the commitments above?").  In the
  * reference nothing ties the proof of encryption's commitment C_y_1 = z*G_y[0] + M1 to the credential proof's C_y[i] = z*G_y[i] + M1:

@@ -55,6 +55,14 @@ struct Error : std::runtime_error {   // a non-zero afx_* return code
 
 typedef std::array<uint8_t, 32> Word;   // a canonical Scalar or a CompressedRistretto
 
+// Symmetric encryption of attributes (src/symmetric.rs): the 30 data bytes, Plaintext (M1, M2, m3), Ciphertext (E1, E2) and the
+// keypair's secret scalars a || a0 || a1, laid out as the C ABI takes them.
+typedef std::array<uint8_t, 30> AttributeData;
+struct Plaintext { Word M1, M2, m3; };
+struct Ciphertext { Word E1, E2; };
+typedef std::array<uint8_t, 96> KeypairSecret;
+static_assert(sizeof(Plaintext) == 96 && sizeof(Ciphertext) == 64 && sizeof(AttributeData) == 30, "C ABI layouts");
+
 // One shape, struct-of-arrays.  fields[f] holds count * 32 bytes.
 struct Batch {
     std::vector<uint8_t> kinds;
@@ -175,8 +183,41 @@ public:
         for (uint8_t x : st) res.push_back(x == 0 ? Result<>::Ok() : Result<>::Err(CredentialError::BadAttribute));
         return {out, res};
     }
+    // Plaintext::from(&[u8; 30]) per item (src/symmetric.rs:135-143); Err(BadAttribute) where no candidate encoding decodes
+    std::pair<std::vector<Plaintext>, std::vector<Result<>>> encode_batch(const std::vector<AttributeData>& data) const {
+        std::vector<Plaintext> out(data.size());
+        std::vector<uint8_t> st(data.size());
+        int rc = afx_encode_plaintexts(ctx_, data.size(), data.empty() ? nullptr : data[0].data(), (uint8_t*)out.data(), st.data());
+        if (rc != AFX_OK) throw Error(rc);
+        return {out, status_results(st, CredentialError::BadAttribute)};
+    }
+    // Keypair::encrypt per item (src/symmetric.rs:252-261); Err(BadAttribute) for a Plaintext the Rust type could never hold
+    std::pair<std::vector<Ciphertext>, std::vector<Result<>>> encrypt_batch(const KeypairSecret& keypair, const std::vector<Plaintext>& pts) const {
+        std::vector<Ciphertext> out(pts.size());
+        std::vector<uint8_t> st(pts.size());
+        int rc = afx_encrypt(ctx_, keypair.data(), pts.size(), (const uint8_t*)pts.data(), (uint8_t*)out.data(), st.data());
+        if (rc != AFX_OK) throw Error(rc);
+        return {out, status_results(st, CredentialError::BadAttribute)};
+    }
+    // Keypair::decrypt per item (src/symmetric.rs:273-289): the data and the Plaintext, or Err(UndecryptableAttribute)
+    std::pair<std::vector<std::pair<AttributeData, Plaintext>>, std::vector<Result<>>> decrypt_batch(const KeypairSecret& keypair,
+                                                                                                       const std::vector<Ciphertext>& cts) const {
+        std::vector<AttributeData> data(cts.size());
+        std::vector<Plaintext> pts(cts.size());
+        std::vector<uint8_t> st(cts.size());
+        int rc = afx_decrypt(ctx_, keypair.data(), cts.size(), (const uint8_t*)cts.data(), (uint8_t*)data.data(), (uint8_t*)pts.data(), st.data());
+        if (rc != AFX_OK) throw Error(rc);
+        std::vector<std::pair<AttributeData, Plaintext>> out;
+        for (size_t i = 0; i < cts.size(); i++) out.push_back({data[i], pts[i]});
+        return {out, status_results(st, CredentialError::UndecryptableAttribute)};
+    }
 
 private:
+    static std::vector<Result<>> status_results(const std::vector<uint8_t>& st, CredentialError e) {
+        std::vector<Result<>> r;
+        for (uint8_t x : st) r.push_back(x == 0 ? Result<>::Ok() : Result<>::Err(e));
+        return r;
+    }
     static std::vector<Result<>> to_results(const std::vector<uint8_t>& v) {
         std::vector<Result<>> r;
         for (uint8_t x : v) r.push_back(x == 0 ? Result<>::Ok() : Result<>::Err(CredentialError::VerificationFailure));
