@@ -936,7 +936,8 @@ AFX_HD u32 ctab_entry_job(const u32* enc /*8 words*/, u32 m, u32* out /*24 words
 
 // ---- primitive self-test (parity hooks for the field / group / scalar code, independent of the protocol flows) ------
 enum : u32 { PRIM_DECOMPRESS_COMPRESS = 0, PRIM_FROM_UNIFORM = 1, PRIM_SCALARMULT = 2, PRIM_WIDE_REDUCE = 3, PRIM_SC_MULADD = 4,
-             PRIM_FE_MUL = 5, PRIM_FE_SQ = 6, PRIM_FE_ADD = 7, PRIM_FE_SUB = 8, PRIM_FE_CHAIN = 9, PRIM_LADDER_STEP = 10, PRIM_RECODE4096 = 11 };
+             PRIM_FE_MUL = 5, PRIM_FE_SQ = 6, PRIM_FE_ADD = 7, PRIM_FE_SUB = 8, PRIM_FE_CHAIN = 9, PRIM_LADDER_STEP = 10, PRIM_RECODE4096 = 11,
+             PRIM_RECODE65536 = 12 };
 // in/out are [count][words][8] item-major.  Returns per item ok (1) / rejected encoding (0) in flags.
 //   0: in 1 word (encoding)          -> out 1 word: compress(decompress(in)); flag = decodes
 //   1: in 2 words (64 uniform bytes) -> out 1 word: compress(from_uniform_bytes(in))
@@ -950,6 +951,9 @@ enum : u32 { PRIM_DECOMPRESS_COMPRESS = 0, PRIM_FROM_UNIFORM = 1, PRIM_SCALARMUL
 //         (gc_dbl4 / gc_add_pn_inl / gc_to_ge) that k_ladders and k_msm_ct use
 //  11: in 1 word (a 256-bit integer)   -> out 1 word: sum_j digit_j * 4096^j mod 2^256 of its biased radix-4096 recoding
 //         (sc_bias4096 / sc_digit4096); equals the input for every input below 2^256 - 2^252; flag = every |digit| <= 2048
+//  12: in 1 word (a 256-bit integer)   -> out 1 word: sum_j digit_j * 65536^j mod 2^256 of its biased radix-2^16 recoding
+//         (sc_bias65536 / sc_digit65536); equals the input for every input below 2^256 - 2^240; flag = every low digit within
+//         [-32768, 32767] and the top digit at most 2^13 + 1
 AFX_HD void primitive_job(u32 op, const u32* in, u32* out, u32* flags, u32 item) {
     u32 w[8]; u32 ok = 1;
     if (op == PRIM_DECOMPRESS_COMPRESS) {
@@ -984,14 +988,16 @@ AFX_HD void primitive_job(u32 op, const u32* in, u32* out, u32* flags, u32 item)
         else if (op == PRIM_FE_SUB) r = fe_sub(a, b);
         else { fe d = fe_sub(a, b); r = fe_add(fe_mul(fe_sq(fe_mul(fe_add(a, b), d)), d), a); }
         fe_to_bytes_words(w, r);
-    } else if (op == PRIM_RECODE4096) {
+    } else if (op == PRIM_RECODE4096 || op == PRIM_RECODE65536) {
+        const bool wide = op == PRIM_RECODE65536;
         sc a; for (int i = 0; i < 8; i++) a.v[i] = in[(size_t)item * 8 + i];
-        u32 rec[8]; sc_bias4096(rec, a);
+        u32 rec[8];
+        if (wide) sc_bias65536(rec, a); else sc_bias4096(rec, a);
         for (int i = 0; i < 8; i++) w[i] = 0;
-        for (int j = 0; j < 22; j++) {
-            int dig = sc_digit4096(rec, 1, j);
-            ok &= (u32)(dig >= -2048 && dig <= 2048);
-            const u32 bit = 12u * (u32)j, w0 = bit >> 5;
+        for (int j = 0; j < (wide ? 16 : 22); j++) {
+            int dig = wide ? sc_digit65536(rec, 1, j) : sc_digit4096(rec, 1, j);
+            ok &= wide ? (u32)(j < 15 ? dig >= -32768 && dig <= 32767 : dig <= 8193) : (u32)(dig >= -2048 && dig <= 2048);
+            const u32 bit = (wide ? 16u : 12u) * (u32)j, w0 = bit >> 5;
             const long long v = (long long)dig * (long long)(1ull << (bit & 31u));
             const u32 ext = v < 0 ? 0xffffffffu : 0u;
             u64 c = 0;

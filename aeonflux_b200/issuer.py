@@ -475,7 +475,8 @@ class Issuer:
             ctypes.memset(kp, 0, 96)
 
     PRIMITIVES = {"decompress_compress": (0, 32), "from_uniform": (1, 64), "scalarmult": (2, 64), "wide_reduce": (3, 64), "sc_muladd": (4, 96),
-                  "fe_mul": (5, 64), "fe_sq": (6, 64), "fe_add": (7, 64), "fe_sub": (8, 64), "fe_chain": (9, 64), "ladder_scalarmult": (10, 64), "recode4096": (11, 32)}
+                  "fe_mul": (5, 64), "fe_sq": (6, 64), "fe_add": (7, 64), "fe_sub": (8, 64), "fe_chain": (9, 64), "ladder_scalarmult": (10, 64), "recode4096": (11, 32),
+                  "recode65536": (12, 32)}
 
     def selftest_primitive(self, name, inputs):
         """Run one field/group/scalar primitive of the engine over raw inputs (uint8 [count][in_bytes]) -> (out [count][32], ok [count])."""

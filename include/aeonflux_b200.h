@@ -350,7 +350,10 @@ int afx_stream_times(const afx_stream* stream, double* fill_s, double* submit_s,
  *   op 9: same inputs                           -> canonical ((a+b)(a-b))^2 (a-b) + a     (chained unreduced intermediates)
  *   op 10: in [count][2][32] scalar, encoding   -> compress(scalar * point) through the completed-coordinates ladder forms
  *   op 11: in [count][32] a 256-bit integer     -> the integer recomposed from its biased radix-4096 digits (the recoding of the
- *                                                  constant-base terms); ok = every digit within [-2048, 2048] */
+ *                                                  constant-base terms); ok = every digit within [-2048, 2048]
+ *   op 12: in [count][32] a 256-bit integer     -> the integer recomposed from its biased radix-2^16 digits (the recoding of the
+ *                                                  constant-base terms with the wide tables); ok = every low digit within
+ *                                                  [-32768, 32767] and the top digit at most 2^13 + 1 */
 int afx_selftest_primitive(afx_ctx* ctx, int op, const uint8_t* in, size_t count, uint8_t* out, uint8_t* ok);
 
 /* Number of kernels this library launched on behalf of `ctx` so far (bench.py's gpu_launches). */
