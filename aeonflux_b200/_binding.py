@@ -38,7 +38,7 @@ class Binding:
                "afx_issue_wire", "afx_show_wire", "afx_presentation_linked_num_commitments", "afx_verify_presentations_linked",
                "afx_verify_presentations_linked_wire", "afx_show_linked", "afx_show_linked_wire", "afx_issuance_batchable_num_fields", "afx_verify_issuances_batchable", "afx_verify_issuances_batchable_rlc", "afx_get_rlc_stats",
                "afx_encode_plaintexts", "afx_encrypt", "afx_decrypt", "afx_encode_plaintexts_device", "afx_encrypt_device",
-               "afx_decrypt_device"]
+               "afx_decrypt_device", "afx_derive_keypairs", "afx_derive_keypairs_device"]
 
     def __init__(self, cdll):
         L = self.L = cdll
@@ -119,6 +119,10 @@ class Binding:
         L.afx_encrypt_device.argtypes = [vp, vp, sz, vp, vp, vp, vp]
         L.afx_decrypt_device.restype = ctypes.c_int
         L.afx_decrypt_device.argtypes = [vp, vp, sz, vp, vp, vp, vp, vp]
+        L.afx_derive_keypairs.restype = ctypes.c_int
+        L.afx_derive_keypairs.argtypes = [vp, sz, vp, vp]
+        L.afx_derive_keypairs_device.restype = ctypes.c_int
+        L.afx_derive_keypairs_device.argtypes = [vp, sz, vp, vp, vp]
         L.afx_selftest_primitive.restype = ctypes.c_int
         L.afx_selftest_primitive.argtypes = [vp, ctypes.c_int, vp, sz, vp, vp]
         L.afx_launch_count.restype = ctypes.c_uint64

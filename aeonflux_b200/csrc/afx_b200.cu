@@ -308,6 +308,11 @@ __global__ void __launch_bounds__(128) k_decrypt(const u32* ct, const u32* kp, u
     u32 item = blockIdx.x * blockDim.x + threadIdx.x;
     if (item < count) decrypt_job(ct, kp, tabs, data, pt, status, count, item_major, item);
 }
+// Keypair::derive: the three hashes and wide reductions, one thread per item (engine.cuh:keypair_scalars_job); pk is compile_keypair
+__global__ void __launch_bounds__(128) k_keypair_scalars(const u32* ms, u32* rows, u32 count) {
+    u32 item = blockIdx.x * blockDim.x + threadIdx.x;
+    if (item < count) keypair_scalars_job(ms, rows, count, item);
+}
 __global__ void k_secret_setup(const u32* secsc, u32 nsec, u32* secdig, const u32* Wenc, u32* W_pniels, u32* bad) {
     u32 t = blockIdx.x * blockDim.x + threadIdx.x;
     if (t < nsec) {
@@ -548,6 +553,9 @@ static void be_launch_encode(const uint8_t* data, u32* pt, uint8_t* status, u32 
 }
 static void be_launch_decrypt(const u32* ct, const u32* kp, u32* tabs, uint8_t* data, u32* pt, uint8_t* status, u32 count, bool item_major, be_stream s) {
     k_decrypt<<<grid_for(count, 128, 1), 128, 0, s>>>(ct, kp, tabs, data, pt, status, count, item_major);
+}
+static void be_launch_keypair_scalars(const u32* ms, u32* rows, u32 count, be_stream s) {
+    k_keypair_scalars<<<grid_for(count, 128, 1), 128, 0, s>>>(ms, rows, count);
 }
 
 #include "api_impl.inc"

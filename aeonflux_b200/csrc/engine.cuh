@@ -1055,8 +1055,9 @@ AFX_HD void comb_entry_job(const u32* enc /*8 words*/, u32 i, u32 e, u32* out /*
     store_fe(out + 16, fe_mul(fe_mul(x, y), FE_D2()));
 }
 
-// ---- symmetric encryption of attributes (encoding.rs:56-82, symmetric.rs:89-96,135-143,252-261,273-289) --------------------------
+// ---- symmetric encryption of attributes (encoding.rs:56-82, symmetric.rs:89-96,135-143,197-215,252-261,273-289) ------------------
 // Keypair::encrypt is a program of the prover stages (program.hpp:compile_encrypt); encoding and decryption are one thread per item.
+// Keypair::derive is one thread per item for its hashes (keypair_scalars_job) and a program for pk (program.hpp:compile_keypair).
 // Word w of the nw words of an item: item-major [count][nw][8] (the host calls) or struct-of-arrays [nw][count][8] (the *_device calls).
 AFX_HD size_t sym_word(u32 count, u32 nw, u32 item_major, u32 w, u32 item) {
     return (item_major ? (size_t)item * nw + w : (size_t)w * count + item) * 8;
@@ -1156,6 +1157,24 @@ AFX_HD void decrypt_job(const u32* ct, const u32* kp, u32* tabs, uint8_t* data, 
         if (pt) for (u32 k = 0; k < 3; k++) store8(pt + sym_word(count, 3, item_major, k, item), w);
     }
     status[item] = (uint8_t)(ok ^ 1u);
+}
+
+// The scalars of Keypair::derive (symmetric.rs:197-215): a = SHA-512(master secret), a0 = SHA-512(a), a1 = SHA-512(a0), each reduced
+// wide mod l.  ms = [count][64] master secrets; rows = the struct-of-arrays rows [3][count][8] a, a0, a1, the fields of
+// program.hpp:compile_keypair, whose comb computes pk.  No branch and no address depends on the master secret.
+AFX_HD void keypair_scalars_job(const u32* ms, u32* rows, u32 count, u32 item) {
+    msg64 m;
+    load8(m.w, ms + (size_t)item * 16);
+    load8(m.w + 8, ms + (size_t)item * 16 + 8);
+#if defined(__CUDA_ARCH__)
+#pragma unroll 1
+#endif
+    for (u32 k = 0; k < 3; k++) {
+        const digest64 h = sha512_words(m, k == 0 ? 16u : 8u);
+        const sc s = sc_reduce512(h.w);
+        store8(rows + ((size_t)k * count + item) * 8, s.v);
+        for (int i = 0; i < 8; i++) { m.w[i] = s.v[i]; m.w[8 + i] = 0; }
+    }
 }
 
 }  // namespace afx

@@ -827,4 +827,18 @@ inline ShapeProgram compile_encrypt() {
     return P;
 }
 
+// Keypair::derive (symmetric.rs:197-215) as a program: pk = a*G_a + a0*G_a0 + a1*G_a1 over the context's system parameters, one MSM of
+// constant bases with secret scalars, which mark_comb_jobs puts on the radix-16 comb (constant-address scans).
+// Fields: a, a0, a1, the rows the hashes of keypair_scalars_job (engine.cuh) leave.  Output words: a, a0, a1, pk -- the 128-byte
+// keypair afx_show takes.
+inline ShapeProgram compile_keypair(const IssuerConsts& ic) {
+    ShapeProgram P; P.is_issue = true;
+    P.n_fields = 3;
+    MsmBuilder m(0); m.con(ic.id_Ga(), sc_field(0)); m.con(ic.id_Ga0(), sc_field(1)); m.con(ic.id_Ga1(), sc_field(2)); P.msms.push_back(m.d);
+    P.n_msm = 1; P.n_proofs = 0;
+    for (u32 k = 0; k < 4; k++) { OutWord o; o.kind = (u16)(k < 3 ? OW_FIELD : OW_COMMIT); o.a = (u16)(k < 3 ? k : 0); o.b = o.c = 0; P.out_words.push_back(o); }
+    mark_comb_jobs(P);
+    return P;
+}
+
 }  // namespace afx

@@ -1,5 +1,6 @@
-// SHA-512 (FIPS 180-4) of the 30 data bytes of an attribute: the hash Plaintext::from (symmetric.rs:135-143) and Keypair::decrypt
-// (symmetric.rs:273-289) apply.  30 bytes fit one padded block.
+// SHA-512 (FIPS 180-4) of messages that fit one padded block: the 30 data bytes of an attribute, which Plaintext::from
+// (symmetric.rs:135-143) and Keypair::decrypt (symmetric.rs:273-289) hash, and the 64-byte master secret and 32-byte scalars that
+// Keypair::derive (symmetric.rs:197-215) hashes.
 #pragma once
 #include "ge.cuh"
 
@@ -9,11 +10,9 @@ AFX_HD u64 rotr64(u64 x, int n) { return (x >> n) | (x << (64 - n)); }
 AFX_HD u32 bswap32(u32 x) { return (x >> 24) | ((x >> 8) & 0xff00u) | ((x << 8) & 0xff0000u) | (x << 24); }
 
 struct digest64 { u32 w[16]; };     // the 64 digest bytes as little-endian words (the form sc_reduce512 and ge_from_uniform take)
-// The message is bytes 1..30 of the 32-byte string msg: where the data sits in its candidate group encodings 2i || data || j
-// (encoding.rs:56-70) and in the compressed M1 a decryption recovers (encoding.rs:75-82).  Passing the words keeps the message
-// in registers.
-AFX_NI digest64 sha512_30(enc32 msg) {
-    const u32 len = 30;
+// The compression function over the one padded block W (16 big-endian words: message, 0x80, zeros, 128-bit bit length), from the
+// initial hash value.  The message builders below are its only callers.
+AFX_HD digest64 sha512_block(u64 W[16]) {
     const u64 K[80] = {
         0x428a2f98d728ae22ull, 0x7137449123ef65cdull, 0xb5c0fbcfec4d3b2full, 0xe9b5dba58189dbbcull, 0x3956c25bf348b538ull,
         0x59f111f1b605d019ull, 0x923f82a4af194f9bull, 0xab1c5ed5da6d8118ull, 0xd807aa98a3030242ull, 0x12835b0145706fbeull,
@@ -31,21 +30,6 @@ AFX_NI digest64 sha512_30(enc32 msg) {
         0xd186b8c721c0c207ull, 0xeada7dd6cde0eb1eull, 0xf57d4f7fee6ed178ull, 0x06f067aa72176fbaull, 0x0a637dc5a2c898a6ull,
         0x113f9804bef90daeull, 0x1b710b35131c471bull, 0x28db77f523047d84ull, 0x32caab7b40c72493ull, 0x3c9ebe0a15c9bebcull,
         0x431d67c49c100d4cull, 0x4cc5d4becb3e42b6ull, 0x597f299cfc657e2aull, 0x5fcb6fab3ad6faecull, 0x6c44198c4a475817ull};
-    // the padded block as 16 big-endian words: message, 0x80, zeros, 128-bit bit length
-    u64 W[16];
-#if defined(__CUDA_ARCH__)
-#pragma unroll
-#endif
-    for (int t = 0; t < 16; t++) {
-        u64 w = 0;
-        for (int b = 0; b < 8; b++) {
-            const u32 i = 8u * (u32)t + (u32)b;
-            const u64 byte = i < len ? (msg.w[(i + 1) >> 2] >> (8 * ((i + 1) & 3))) & 0xffu : i == len ? 0x80u : 0u;
-            w = (w << 8) | byte;
-        }
-        W[t] = w;
-    }
-    W[15] |= (u64)len * 8u;
     u64 H[8] = {0x6a09e667f3bcc908ull, 0xbb67ae8584caa73bull, 0x3c6ef372fe94f82bull, 0xa54ff53a5f1d36f1ull,
                 0x510e527fade682d1ull, 0x9b05688c2b3e6c1full, 0x1f83d9abfb41bd6bull, 0x5be0cd19137e2179ull};
     u64 a = H[0], b = H[1], c = H[2], d = H[3], e = H[4], f = H[5], g = H[6], h = H[7];
@@ -73,6 +57,45 @@ AFX_NI digest64 sha512_30(enc32 msg) {
         out.w[2 * i + 1] = bswap32((u32)H[i]);
     }
     return out;
+}
+
+// The message is bytes 1..30 of the 32-byte string msg: where the data sits in its candidate group encodings 2i || data || j
+// (encoding.rs:56-70) and in the compressed M1 a decryption recovers (encoding.rs:75-82).  Passing the words keeps the message
+// in registers.
+AFX_NI digest64 sha512_30(enc32 msg) {
+    const u32 len = 30;
+    u64 W[16];
+#if defined(__CUDA_ARCH__)
+#pragma unroll
+#endif
+    for (int t = 0; t < 16; t++) {
+        u64 w = 0;
+        for (int b = 0; b < 8; b++) {
+            const u32 i = 8u * (u32)t + (u32)b;
+            const u64 byte = i < len ? (msg.w[(i + 1) >> 2] >> (8 * ((i + 1) & 3))) & 0xffu : i == len ? 0x80u : 0u;
+            w = (w << 8) | byte;
+        }
+        W[t] = w;
+    }
+    W[15] |= (u64)len * 8u;
+    return sha512_block(W);
+}
+
+struct msg64 { u32 w[16]; };        // up to 64 message bytes as little-endian words
+// The message is the first 4 * nw bytes of m, nw = 16 (a master secret) or 8 (a scalar's 32 bytes).  nw is public: it selects where
+// the padding starts, never a message byte.  Passing the words keeps the message in registers.
+AFX_NI digest64 sha512_words(msg64 m, u32 nw) {
+    u64 W[16];
+#if defined(__CUDA_ARCH__)
+#pragma unroll
+#endif
+    for (int t = 0; t < 16; t++) {
+        const u32 k = 2u * (u32)t;
+        const u64 word = ((u64)bswap32(m.w[k & 15]) << 32) | bswap32(m.w[(k + 1) & 15]);
+        W[t] = k < nw ? word : k == nw ? 0x8000000000000000ull : 0u;
+    }
+    W[15] |= (u64)nw * 32u;
+    return sha512_block(W);
 }
 
 }  // namespace afx

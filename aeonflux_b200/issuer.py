@@ -474,6 +474,24 @@ class Issuer:
         finally:
             ctypes.memset(kp, 0, 96)
 
+    def derive_keypairs(self, master_secrets, out=None):
+        """Keypair::derive (symmetric.rs:197-215) of every 64-byte master secret (uint8 [count][64]) under this context's system
+        parameters -> keypairs uint8 [count][128]: a || a0 || a1 || pk, the keypair show takes (its first 96 bytes are what
+        encrypt and decrypt take).  Keypair::generate is this applied to 64 rng bytes."""
+        ms = np.asarray(master_secrets, dtype=np.uint8)
+        if ms.ndim != 2 or ms.shape[1] != 64:
+            raise ValueError("master_secrets must be [count][64] bytes")
+        ms = np.ascontiguousarray(ms)
+        count = ms.shape[0]
+        out = np.zeros((count, 128), np.uint8) if out is None else self._array("out", out, (count, 128))
+        self._b.check(self._b.L.afx_derive_keypairs(self._h, count, ms.ctypes.data, out.ctypes.data))
+        return out
+
+    def derive_keypairs_device(self, count, master_secrets_dev_ptr, keypairs_dev_ptr, stream=0):
+        """Enqueue derive_keypairs on device memory: master secrets [count][64] -> keypairs [4][count][32] (the a, a0, a1, pk rows
+        show_batch_device takes); count <= max_batch, no synchronisation."""
+        self._b.check(self._b.L.afx_derive_keypairs_device(self._h, count, master_secrets_dev_ptr, keypairs_dev_ptr, stream))
+
     PRIMITIVES = {"decompress_compress": (0, 32), "from_uniform": (1, 64), "scalarmult": (2, 64), "wide_reduce": (3, 64), "sc_muladd": (4, 96),
                   "fe_mul": (5, 64), "fe_sq": (6, 64), "fe_add": (7, 64), "fe_sub": (8, 64), "fe_chain": (9, 64), "ladder_scalarmult": (10, 64), "recode4096": (11, 32),
                   "recode65536": (12, 32)}

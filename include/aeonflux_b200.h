@@ -274,6 +274,24 @@ int afx_encrypt_device(afx_ctx* ctx, const uint8_t keypair[96], size_t count, co
 int afx_decrypt_device(afx_ctx* ctx, const uint8_t keypair[96], size_t count, const void* ciphertexts_dev, void* data_dev,
                        void* plaintexts_dev, void* status_dev, void* stream);
 
+/* Batch Keypair::derive (src/symmetric.rs:197-215): from each 64-byte master secret,
+ *     a = SHA-512(master_secret) mod l,  a0 = SHA-512(a) mod l,  a1 = SHA-512(a0) mod l,  pk = a*G_a + a0*G_a0 + a1*G_a1
+ * (wide reductions; G_a, G_a0, G_a1 of the context's SystemParameters, so the same master secret gives different keypairs under
+ * different issuers).  Keypair::generate (src/symmetric.rs:227-241) is this call applied to 64 bytes of rng output: as with
+ * afx_issue and afx_show the caller supplies the rng bytes, and they are the master secret generate returns.  The call needs no
+ * issuer secret (a context created with secret = NULL suffices).  Every 64-byte string derives a keypair: there is no status.
+ *   master_secrets = [count][64] bytes
+ *   keypairs       = [count][128] bytes a || a0 || a1 || pk: exactly the keypair afx_show takes, whose first 96 bytes are the keypair
+ *                    afx_encrypt and afx_decrypt take.  Runs in passes of max_batch items.
+ * The device form takes device memory: master_secrets_dev = [count][64], keypairs_dev = [4][count][32], the rows a, a0, a1, pk --
+ * the four keypair rows of afx_show_device's input, so they can be handed over without a host round trip.  count <= max_batch;
+ * enqueued on `stream` (a cudaStream_t; NULL = default stream) without synchronizing.
+ * Timing: the hashes run one thread per item with no branch or address depending on the master secret, and pk is a comb over the
+ * three generators with constant-address table scans.  The device copies of the master secrets and of a, a0, a1 the call makes are
+ * zeroed on the stream at the end of every pass. */
+int afx_derive_keypairs(afx_ctx* ctx, size_t count, const uint8_t* master_secrets, uint8_t* keypairs);
+int afx_derive_keypairs_device(afx_ctx* ctx, size_t count, const void* master_secrets_dev, void* keypairs_dev, void* stream);
+
 /* Linked presentations (opt-in; NOT the reference's protocol but the fix its authors left as a TODO: README.md:119-122,
  * src/nizk/presentation.rs:292 "don't we also need DLEQ between the plaintext here and that in the commitments above?").  In the
  * reference nothing ties the proof of encryption's commitment C_y_1 = z*G_y[0] + M1 to the credential proof's C_y[i] = z*G_y[i] + M1:

@@ -21,6 +21,7 @@
 #define AEONFLUX_B200_HPP
 
 #include <array>
+#include <cstddef>
 #include <cstdint>
 #include <cstring>
 #include <stdexcept>
@@ -62,6 +63,11 @@ struct Plaintext { Word M1, M2, m3; };
 struct Ciphertext { Word E1, E2; };
 typedef std::array<uint8_t, 96> KeypairSecret;
 static_assert(sizeof(Plaintext) == 96 && sizeof(Ciphertext) == 64 && sizeof(AttributeData) == 30, "C ABI layouts");
+// Keypair::derive's input and output (src/symmetric.rs:74-79,197-215): the 64-byte master secret, and a || a0 || a1 || pk -- the
+// keypair afx_show takes, whose first 96 bytes (secret) are what encrypt_batch and decrypt_batch take.
+typedef std::array<uint8_t, 64> MasterSecret;
+struct Keypair { KeypairSecret secret; Word pk; };
+static_assert(sizeof(MasterSecret) == 64 && sizeof(Keypair) == 128 && offsetof(Keypair, pk) == 96, "C ABI layouts");
 
 // One shape, struct-of-arrays.  fields[f] holds count * 32 bytes.
 struct Batch {
@@ -198,6 +204,13 @@ public:
         int rc = afx_encrypt(ctx_, keypair.data(), pts.size(), (const uint8_t*)pts.data(), (uint8_t*)out.data(), st.data());
         if (rc != AFX_OK) throw Error(rc);
         return {out, status_results(st, CredentialError::BadAttribute)};
+    }
+    // Keypair::derive per item (src/symmetric.rs:197-215) under this issuer's system parameters; Keypair::generate is this on 64 rng bytes
+    std::vector<Keypair> derive_keypairs(const std::vector<MasterSecret>& master_secrets) const {
+        std::vector<Keypair> out(master_secrets.size());
+        int rc = afx_derive_keypairs(ctx_, master_secrets.size(), master_secrets.empty() ? nullptr : master_secrets[0].data(), (uint8_t*)out.data());
+        if (rc != AFX_OK) throw Error(rc);
+        return out;
     }
     // Keypair::decrypt per item (src/symmetric.rs:273-289): the data and the Plaintext, or Err(UndecryptableAttribute)
     std::pair<std::vector<std::pair<AttributeData, Plaintext>>, std::vector<Result<>>> decrypt_batch(const KeypairSecret& keypair,
