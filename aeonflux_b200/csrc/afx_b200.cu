@@ -130,6 +130,14 @@ __global__ void __launch_bounds__(128) k_amac_combine(Workspace ws, const AmacDe
     if (item < ws.count) amac_combine_job(ws, *d, parts, n_parts, item);
 }
 
+// Commitment encodings of the verify MSMs (engine.cuh:commit_encode_job): thread (item, y) encodes entries [y * per, y * per + per)
+// of the slot list under one inversion
+__global__ void __launch_bounds__(128) k_commit_encode(Workspace ws, const u32* slots, u32 nslots, u32 per) {
+    u32 item = blockIdx.x * blockDim.x + threadIdx.x;
+    const u32 lo = blockIdx.y * per;
+    if (item < ws.count) commit_encode_job(ws, slots + lo, nslots - lo < per ? nslots - lo : per, item);
+}
+
 // Issuer::issue: the same per-(item, job) ladders with every lookup constant-address (all scalars are secrets)
 __global__ void __launch_bounds__(TPB_MSM, AFX_MSM_MINB) k_msm_ct(Workspace ws, const MsmDesc* msms, const u32* group_idx) {
     extern __shared__ __align__(16) u32 smem[];
@@ -484,6 +492,9 @@ static void be_launch_ladders_parts(const Workspace& ws, const AmacDesc* amac, c
 }
 static void be_launch_amac_combine(const Workspace& ws, const AmacDesc* amac, const u32* parts_out, u32 n_parts, be_stream s) {
     k_amac_combine<<<grid_for(ws.count, 128, 1), 128, 0, s>>>(ws, amac, parts_out, n_parts);
+}
+static void be_launch_commit_encode(const Workspace& ws, const u32* d_slots, u32 nslots, u32 per, be_stream s) {
+    k_commit_encode<<<grid_for(ws.count, 128, (nslots + per - 1) / per), 128, 0, s>>>(ws, d_slots, nslots, per);
 }
 static void be_launch_msm_ct(const Workspace& ws, const MsmDesc* d_msms, const u32* d_idx, u32 nidx, u32 max_terms, be_stream s) {
     const auto [tpb, smem] = ladder_geometry(max_terms);

@@ -142,6 +142,7 @@ struct Workspace {
     const u64* lanes;    // transcript block masks
     const TxHole* holes;
     const TxIdCheck* idchecks;
+    u32* commit_q;       // [n_msm][count][32]  verify MSMs: Q = R/2 in extended coordinates, which commit_encode_job encodes into commit
 };
 
 enum : u32 { ST_BAD_POINT = 1, ST_BAD_SCALAR = 2, ST_IDENTITY = 4, ST_CHALLENGE = 8 };
@@ -225,6 +226,7 @@ AFX_HD u32* atab_ptr(const Workspace& ws, u32 slot, u32 item) {
 AFX_HD u32* ext_ptr(const Workspace& ws, u32 slot, u32 item) { return ws.ext + ((size_t)slot * ws.count + item) * 32; }
 AFX_HD u32* comp_ptr(const Workspace& ws, u32 slot, u32 item) { return ws.comp + ((size_t)slot * ws.count + item) * 8; }
 AFX_HD u32* commit_ptr(const Workspace& ws, u32 slot, u32 item) { return ws.commit + ((size_t)slot * ws.count + item) * 8; }
+AFX_HD u32* commit_q_ptr(const Workspace& ws, u32 slot, u32 item) { return ws.commit_q + ((size_t)slot * ws.count + item) * 32; }
 
 AFX_HD void status_or(const Workspace& ws, u32 item, u32 bits) {
 #if defined(__CUDA_ARCH__)
@@ -479,6 +481,8 @@ struct CtabResolver {
 };
 
 // ---- stage: msm -----------------------------------------------------------------------------------------------
+// Every scalar is halved mod l, so the job computes Q = R/2 of the constraint's R = sum s_j * P_j and leaves it in commit_q in
+// extended coordinates: commit_encode_job then encodes 2Q, which needs one inversion per item instead of a square root per job.
 // scratch: (nvar + ncon) * 8 words per item of recoded scalars.  ctab_of(k) returns the table base of constant term k
 // (global memory).
 template <typename CtabOf>
@@ -487,7 +491,7 @@ AFX_HD void msm_job(const Workspace& ws, const MsmDesc& d, u32 item, u32* scratc
         gc cacc = gc_identity();
         for (u32 k = 0; k < d.ncon; k++) {
             u32 rec[8];
-            sc_recode16(rec, eval_scalar(ws, d.con[k].s, item));
+            sc_recode16(rec, sc_half(eval_scalar(ws, d.con[k].s, item)));
             const u32* comb = ws.comb + (size_t)d.con[k].ctab * COMB_WINDOWS * COMB_ENTRIES * 24;
             for (int i = 0; i < COMB_WINDOWS; i++) {
                 int dig = sc_digit16(rec, i);
@@ -499,20 +503,19 @@ AFX_HD void msm_job(const Workspace& ws, const MsmDesc& d, u32 item, u32* scratc
                 }
             }
         }
-        u32 w[8];
-        ge_compress(w, gc_to_ge(cacc));
-        if (active) store8(commit_ptr(ws, d.out_slot, item), w);
+        if (active) store_ge(commit_q_ptr(ws, d.out_slot, item), gc_to_ge(cacc));
         return;
     }
     const bool wide = ws.ctabs16 != nullptr;      // radix-2^16 constant tables: a digit every 4th window instead of every 3rd
     for (u32 k = 0; k < d.nvar; k++) {
         u32 rec[8];
-        sc_recode16(rec, eval_scalar(ws, d.var[k].s, item));
+        sc_recode16(rec, sc_half(eval_scalar(ws, d.var[k].s, item)));
         for (int w = 0; w < 8; w++) scratch[(k * 8 + w) * scratch_stride] = rec[w];
     }
     for (u32 k = 0; k < d.ncon; k++) {
         u32 rec[8];
-        if (wide) sc_bias65536(rec, eval_scalar(ws, d.con[k].s, item)); else sc_bias4096(rec, eval_scalar(ws, d.con[k].s, item));
+        const sc h = sc_half(eval_scalar(ws, d.con[k].s, item));
+        if (wide) sc_bias65536(rec, h); else sc_bias4096(rec, h);
         for (int w = 0; w < 8; w++) scratch[((d.nvar + k) * 8 + w) * scratch_stride] = rec[w];
     }
     gc cacc = gc_identity();
@@ -551,9 +554,33 @@ AFX_HD void msm_job(const Workspace& ws, const MsmDesc& d, u32 item, u32* scratc
             }
         }
     }
-    u32 w[8];
-    ge_compress(w, gc_to_ge(cacc));
-    if (active) store8(commit_ptr(ws, d.out_slot, item), w);
+    if (active) store_ge(commit_q_ptr(ws, d.out_slot, item), gc_to_ge(cacc));
+}
+
+// ---- stage: commitment encoding ----------------------------------------------------------------------------------
+// Encodes the verify MSMs' results: commit[slot] = the encoding of 2 * commit_q[slot] for the n slots slots[0 .. n) of one
+// item, with one field inversion for all of them (ge.cuh:dac_begin).  2Q encodes as R: every base of a verify MSM is a decoded
+// point or a sum of such points, so it lies in 2E, and 2Q - R = sum k_j * l * P_j (k_j in {0, 1}) is 4-torsion.  The prefix
+// products of the batch are kept in the commit words they are about to be replaced with.
+AFX_HD void commit_encode_job(const Workspace& ws, const u32* slots, u32 n, u32 item) {
+    fe acc = fe_one();
+    for (u32 k = 0; k < n; k++) {
+        u32 zero;
+        const fe x = dac_den(dac_begin(load_ge(commit_q_ptr(ws, slots[k], item))), zero);
+        store_fe(commit_ptr(ws, slots[k], item), acc);
+        acc = fe_mul(acc, x);
+    }
+    fe inv = fe_invert(acc);
+    for (u32 k = n; k-- > 0;) {
+        u32 zero;
+        const dac_state st = dac_begin(load_ge(commit_q_ptr(ws, slots[k], item)));
+        const fe x = dac_den(st, zero);
+        u32* out = commit_ptr(ws, slots[k], item);
+        const fe inv_k = fe_mul(inv, load_fe(out));
+        inv = fe_mul(inv, x);
+        enc32 e = dac_finish(st, inv_k, zero);
+        store8(out, e.w);
+    }
 }
 
 // ---- stage: constant-schedule msm (Issuer::issue) ----------------------------------------------------------------

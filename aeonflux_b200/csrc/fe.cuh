@@ -356,8 +356,9 @@ AFX_HD fe fe_from_bytes_words(const u32* w) { fe r; for (int i = 0; i < 8; i++) 
 AFX_HD void fe_to_bytes_words(u32* w, const fe& a) { fe c = fe_canonical(a); for (int i = 0; i < 8; i++) w[i] = c.v[i]; }
 
 // ---- addition chains -------------------------------------------------------------------------------
-// x^(2^252 - 3) = x^((p-5)/8): 251 squarings + 11 multiplies, fully in registers.
-AFX_NI fe fe_pow_p58(fe x) {
+// The common head of the two chains below: x^(2^250 - 1) and x^11.  249 squarings + 10 multiplies.
+struct fe_pow250 { fe a250, x11; };
+AFX_HD fe_pow250 fe_pow22501(const fe& x) {
     fe x2 = fe_sq(x);                       // 2
     fe x9 = fe_mul(fe_sqn(x2, 2), x);       // 9
     fe x11 = fe_mul(x9, x2);                // 11
@@ -368,9 +369,13 @@ AFX_NI fe fe_pow_p58(fe x) {
     fe a50 = fe_mul(fe_sqn(a40, 10), a10);  // 2^50 - 1
     fe a100 = fe_mul(fe_sqn(a50, 50), a50); // 2^100 - 1
     fe a200 = fe_mul(fe_sqn(a100, 100), a100); // 2^200 - 1
-    fe a250 = fe_mul(fe_sqn(a200, 50), a50);   // 2^250 - 1
-    return fe_mul(fe_sqn(a250, 2), x);         // 2^252 - 3
+    fe_pow250 r; r.a250 = fe_mul(fe_sqn(a200, 50), a50); r.x11 = x11;   // 2^250 - 1
+    return r;
 }
+// x^(2^252 - 3) = x^((p-5)/8): 251 squarings + 11 multiplies, fully in registers.
+AFX_NI fe fe_pow_p58(fe x) { return fe_mul(fe_sqn(fe_pow22501(x).a250, 2), x); }
+// x^(p-2) = x^(2^255 - 21) = 1/x (0 for x = 0): 254 squarings + 11 multiplies.
+AFX_NI fe fe_invert(fe x) { fe_pow250 t = fe_pow22501(x); return fe_mul(fe_sqn(t.a250, 5), t.x11); }
 
 // sqrt_ratio_i(u, v) (SURVEY A.1): returns was_square, r = the non-negative root of u/v or of i*u/v.
 struct fe_ok { fe r; u32 ok; };

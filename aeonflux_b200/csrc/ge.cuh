@@ -172,6 +172,40 @@ AFX_NI enc32 ge_compress_v(ge p) {
 }
 AFX_HD void ge_compress(u32* out, const ge& p) { enc32 e = ge_compress_v(p); for (int i = 0; i < 8; i++) out[i] = e.w[i]; }
 
+// Encoding of a DOUBLED point, in batches (curve25519-dalek RistrettoPoint::double_and_compress_batch).  For 2Q the square
+// root the encoding needs is a rational function of Q's coordinates, so a batch of doubled points shares one field inversion
+// (Montgomery's trick) where compress() pays an inverse square root per point.  Per point: dac_begin, then dac_den into the
+// batch's running product, then dac_finish with inv = 1 / dac_den.  eg * fh = 0 exactly when 2Q is 4-torsion, whose
+// encoding is the identity's (32 zero bytes): such a factor is replaced by 1 so that it does not zero the whole product.
+struct dac_state { fe e, f, g, h, eg, fh; };
+AFX_NI dac_state dac_begin(ge q) {       // 4S + 4M
+    fe XX = fe_sq(q.X), YY = fe_sq(q.Y), ZZ = fe_sq(q.Z), dTT = fe_mul(FE_D(), fe_sq(q.T));
+    dac_state s;
+    s.e = fe_mul(fe_add(q.X, q.X), q.Y); s.f = fe_add(ZZ, dTT); s.g = fe_add(YY, XX); s.h = fe_sub(ZZ, dTT);
+    s.eg = fe_mul(s.e, s.g); s.fh = fe_mul(s.f, s.h);
+    return s;
+}
+// eg * fh, or 1 when it is zero (zero = 1 then)
+AFX_HD fe dac_den(const dac_state& s, u32& zero) {
+    fe x = fe_mul(s.eg, s.fh);
+    zero = fe_is_zero(x);
+    return fe_select(x, fe_one(), zero);
+}
+// 8 encoding words of 2Q from inv = 1 / dac_den: 8M, all selects, no branch
+AFX_NI enc32 dac_finish(dac_state s, fe inv, u32 zero) {
+    fe z_inv = fe_mul(s.eg, inv), t_inv = fe_mul(s.fh, inv);
+    u32 rotate = fe_is_negative(fe_mul(s.eg, z_inv));
+    fe e = fe_select(s.e, s.g, rotate);
+    fe g = fe_select(s.g, fe_neg(s.e), rotate);
+    fe h = fe_select(s.h, fe_mul(s.f, FE_SQRT_M1()), rotate);
+    fe magic = fe_select(FE_INVSQRT_A_MINUS_D(), FE_SQRT_M1(), rotate);
+    g = fe_cneg(g, fe_is_negative(fe_mul(fe_mul(h, e), z_inv)));
+    fe s_ = fe_abs(fe_mul(fe_sub(h, g), fe_mul(magic, fe_mul(g, t_inv))));
+    s_ = fe_select(s_, fe_zero(), zero);
+    enc32 out; fe_to_bytes_words(out.w, s_);
+    return out;
+}
+
 // Elligator map (RFC 9496 4.3.4 MAP; dalek elligator_ristretto_flavor), SURVEY A.2
 AFX_NI ge ge_elligator(fe r0) {
     fe one = fe_one();

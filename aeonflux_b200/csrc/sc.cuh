@@ -39,6 +39,17 @@ AFX_HD sc sc_neg(const sc& a) {
     return r;
 }
 
+// a * 2^-1 mod l for canonical a: (a + l) / 2 if a is odd, a / 2 otherwise, without a branch.  a + l < 2^254 fits the 8 words.
+AFX_HD sc sc_half(const sc& a) {
+    const u32 m = 0u - (a.v[0] & 1u);
+    u32 t[8]; u64 c = 0;
+    for (int i = 0; i < 8; i++) { c += (u64)a.v[i] + (sc_L(i) & m); t[i] = (u32)c; c >>= 32; }
+    sc r;
+    for (int i = 0; i < 7; i++) r.v[i] = (t[i] >> 1) | (t[i + 1] << 31);
+    r.v[7] = t[7] >> 1;
+    return r;
+}
+
 // x (16 words, < 2^512) mod l.  Barrett, HAC 14.42 with b = 2^32, k = 8.
 AFX_HD sc sc_reduce512(const u32* x) {
     // q2 = (x >> 224) * mu ; only words >= 9 of q2 are needed but low words feed carries
