@@ -38,7 +38,8 @@ class Binding:
                "afx_issue_wire", "afx_show_wire", "afx_presentation_linked_num_commitments", "afx_verify_presentations_linked",
                "afx_verify_presentations_linked_wire", "afx_show_linked", "afx_show_linked_wire", "afx_issuance_batchable_num_fields", "afx_verify_issuances_batchable", "afx_verify_issuances_batchable_rlc", "afx_get_rlc_stats",
                "afx_encode_plaintexts", "afx_encrypt", "afx_decrypt", "afx_encode_plaintexts_device", "afx_encrypt_device",
-               "afx_decrypt_device", "afx_derive_keypairs", "afx_derive_keypairs_device"]
+               "afx_decrypt_device", "afx_derive_keypairs", "afx_derive_keypairs_device", "afx_issue_batchable", "afx_issue_batchable_device",
+               "afx_show_batchable", "afx_show_batchable_device"]
 
     def __init__(self, cdll):
         L = self.L = cdll
@@ -86,16 +87,14 @@ class Binding:
             getattr(L, f).argtypes = [vp, ctypes.c_uint16, ctypes.c_char_p, sz, vp, vp]
         L.afx_request_num_fields.restype = sz
         L.afx_request_num_fields.argtypes = [ctypes.c_uint16]
-        L.afx_issue.restype = ctypes.c_int
-        L.afx_issue.argtypes = [vp, ctypes.POINTER(afx_presentation_batch), ctypes.POINTER(afx_issuance_out), vp, ctypes.POINTER(afx_debug_dump)]
-        L.afx_issue_device.restype = ctypes.c_int
-        L.afx_issue_device.argtypes = [vp, ctypes.c_uint16, ctypes.c_char_p, sz, vp, vp, vp, vp]
         L.afx_show_num_fields.restype = sz
         L.afx_show_num_fields.argtypes = [ctypes.c_uint16, ctypes.c_char_p]
-        L.afx_show.restype = ctypes.c_int
-        L.afx_show.argtypes = [vp, ctypes.POINTER(afx_presentation_batch), ctypes.POINTER(afx_issuance_out), vp, ctypes.POINTER(afx_debug_dump)]
-        L.afx_show_device.restype = ctypes.c_int
-        L.afx_show_device.argtypes = [vp, ctypes.c_uint16, ctypes.c_char_p, sz, vp, vp, vp, vp]
+        for f in ("afx_issue", "afx_show", "afx_issue_batchable", "afx_show_batchable"):
+            getattr(L, f).restype = ctypes.c_int
+            getattr(L, f).argtypes = [vp, ctypes.POINTER(afx_presentation_batch), ctypes.POINTER(afx_issuance_out), vp, ctypes.POINTER(afx_debug_dump)]
+        for f in ("afx_issue_device", "afx_show_device", "afx_issue_batchable_device", "afx_show_batchable_device"):
+            getattr(L, f).restype = ctypes.c_int
+            getattr(L, f).argtypes = [vp, ctypes.c_uint16, ctypes.c_char_p, sz, vp, vp, vp, vp]
         L.afx_presentation_linked_num_commitments.restype = sz
         L.afx_presentation_linked_num_commitments.argtypes = [ctypes.c_uint16, ctypes.c_char_p]
         L.afx_verify_presentations_linked.restype = ctypes.c_int

@@ -539,8 +539,11 @@ inline ShapeProgram compile_issuance_verify(const IssuerConsts& ic, u32 n, const
 // with the rng output supplied by the caller.  kinds: 0 = scalar attribute, 2 = point attribute.
 // Fields: attr[n], then two 32-byte words (the 64 rng bytes) per random value: t, U, blinding[n+5] in the order the
 // witnesses are allocated (w, w', x_0, x_1, y[n], "1"; issuance.rs:52-68).  Output words: t, U, V, challenge, responses[n+5].
+// batchable = the same proof returned as zkp's prove_batchable returns it: the challenge word is replaced by the encodings of the
+// three blinding commitments (constraint order C_W, I, V), n + 11 output words, which with attribute[n] in front is the layout
+// compile_issuance_verify(..., batchable = true) takes.  The transcript and the responses do not change.
 inline size_t issue_num_fields(u32 n) { return (size_t)n + 2 * ((size_t)n + 7); }
-inline ShapeProgram compile_issue(const IssuerConsts& ic, u32 n, const uint8_t* kinds) {
+inline ShapeProgram compile_issue(const IssuerConsts& ic, u32 n, const uint8_t* kinds, bool batchable = false) {
     if (n != ic.n || n == 0 || n > MAX_ATTRS) throw std::invalid_argument("attribute count does not match the issuer's");  // amacs.rs:285-287
     for (u32 i = 0; i < n; i++) if (kinds[i] != 0 && kinds[i] != 2) throw std::invalid_argument("bad request kind");
     ShapeProgram P; P.is_issue = true;
@@ -615,7 +618,9 @@ inline ShapeProgram compile_issue(const IssuerConsts& ic, u32 n, const uint8_t* 
     finish_transcript(P, tb, 0xffff, 0);
     P.n_msm = slot; P.n_proofs = 1;
     auto word = [&](u32 kind, u32 a, u32 b = 0, u32 c = 0) { OutWord o; o.kind = (u16)kind; o.a = (u16)a; o.b = (u16)b; o.c = (u16)c; P.out_words.push_back(o); };
-    word(OW_DERIVED, D_T); word(OW_COMP, C_U); word(OW_COMMIT, S_V); word(OW_CHAL, 0);
+    word(OW_DERIVED, D_T); word(OW_COMP, C_U); word(OW_COMMIT, S_V);
+    if (batchable) for (u32 s : {S_CW, S_I, S_CV}) word(OW_COMMIT, s);
+    else word(OW_CHAL, 0);
     const u32 wit[4] = {sref_secret(2 + n), sref_secret(3 + n), sref_secret(sec_x0()), sref_secret(sec_x1())};   // w, w', x_0, x_1
     for (u32 k = 0; k < 4; k++) word(OW_RESP, 0, wit[k], sref_derived(D_B(k)));
     for (u32 i = 0; i < n; i++) word(OW_RESP, 0, sref_secret(sec_y(i)), sref_derived(D_B(4 + i)));
@@ -631,7 +636,10 @@ inline ShapeProgram compile_issue(const IssuerConsts& ic, u32 n, const uint8_t* 
 // Fields: t, U, V, then per attribute: scalar m_i (kinds 0/1) | point M_i (kind 2) | plaintext M1, M2, m3 (kind 3);
 //         then a, a0, a1, pk of the symmetric keypair (only if some kind is 3); then two 32-byte words (64 rng bytes) per
 //         random value: z, the main proof's 3 + h_s blindings, then 6 blindings per hidden plaintext.
-// Output words: exactly the presentation layout of include/aeonflux_b200.h.
+// Output words: exactly the presentation layout of include/aeonflux_b200.h.  batchable = zkp's prove_batchable: every challenge word
+// is replaced by that proof's blinding commitments in constraint order (main proof: Z, C_x_1, the C_y constraints; proof of
+// encryption: pk, C_y_1-E2, C_y_2', E1, C_y_3), which is the layout compile_presentation(..., batchable = true) takes.  The
+// challenges are still derived: the responses need them.  Like compile_presentation, the linked statement has no batchable form.
 // Every commitment is rewritten over the per-issuer generators and the *input* points (U, M2): e.g. the blinding commitment
 // b_t*C_x_0 + b_z0*G_x_0 + b_z*G_x_1 with C_x_0 = z*G_x_0 + U becomes (b_z0 + b_t*z)*G_x_0 + b_z*G_x_1 + b_t*U, so no ladder
 // has to wait for another ladder's output and every job of an item runs in one launch.
@@ -640,9 +648,10 @@ inline size_t show_num_fields(u32 n, const uint8_t* kinds) {
     for (u32 i = 0; i < n; i++) { f += kinds[i] == 3 ? 3 : 1; hs += kinds[i] == 1; hp += kinds[i] == 3; }
     return f + (hp ? 4 : 0) + 2 + 2 * (3 + hs) + 12 * hp;
 }
-inline ShapeProgram compile_show(const IssuerConsts& ic, u32 n, const uint8_t* kinds, bool linked = false) {
+inline ShapeProgram compile_show(const IssuerConsts& ic, u32 n, const uint8_t* kinds, bool linked = false, bool batchable = false) {
     if (n != ic.n || n == 0 || n > MAX_ATTRS) throw std::invalid_argument("attribute count does not match the issuer's");
     for (u32 i = 0; i < n; i++) if (kinds[i] > 3) throw std::invalid_argument("bad attribute kind");
+    if (batchable && linked) throw std::invalid_argument("the linked statement is only built for compact proofs");
     ShapeProgram P; P.is_issue = true;
     u32 hs = 0, hp = 0; std::vector<int> ss_rank(n, -1);
     for (u32 i = 0; i < n; i++) { if (kinds[i] == 1) ss_rank[i] = (int)hs++; hp += kinds[i] == 3; }
@@ -741,7 +750,8 @@ inline ShapeProgram compile_show(const IssuerConsts& ic, u32 n, const uint8_t* k
         finish_transcript(P, tb, 0xffff, 0);
     }
     auto word = [&](u32 kind, u32 a, u32 b = 0, u32 c = 0) { OutWord o; o.kind = (u16)kind; o.a = (u16)a; o.b = (u16)b; o.c = (u16)c; P.out_words.push_back(o); };
-    word(OW_CHAL, 0);
+    if (batchable) for (const Con& c : main_cons) word(OW_COMMIT, c.slot);
+    else word(OW_CHAL, 0);
     word(OW_RESP, 0, D_z, D_bz); word(OW_RESP, 0, D_z0, D_bz0); word(OW_RESP, 0, F_T, D_bt);
     for (u32 i = 0; i < n; i++) if (kinds[i] == 1) word(OW_RESP, 0, F_ATTR[i], D_bm[ss_rank[i]]);
     word(OW_COMMIT, S_CX0); word(OW_COMMIT, S_CX1); word(OW_COMMIT, S_CV);
@@ -792,7 +802,8 @@ inline ShapeProgram compile_show(const IssuerConsts& ic, u32 n, const uint8_t* k
         for (u32 s2 : {S_Rpk, S_RD, S_RCY2P, S_RE1, S_RCY3}) P.dump_commit.push_back(s2);
         tb.challenge();
         finish_transcript(P, tb, 0xffff, 1 + e);
-        word(OW_CHAL, 1 + e);
+        if (batchable) for (u32 s2 : {S_Rpk, S_RD, S_RCY2P, S_RE1, S_RCY3}) word(OW_COMMIT, s2);
+        else word(OW_CHAL, 1 + e);
         word(OW_RESP, 1 + e, F_A, D_ba); word(OW_RESP, 1 + e, F_A0, D_ba0); word(OW_RESP, 1 + e, F_A1, D_ba1);
         word(OW_RESP, 1 + e, F_M3, D_bm3); word(OW_RESP, 1 + e, D_z, D_bze); word(OW_RESP, 1 + e, D_z1, D_bz1);
         word(OW_FIELD, F_PK);

@@ -22,6 +22,7 @@ import numpy as np
 from . import _binding as B
 
 KIND_PUBLIC_SCALAR, KIND_SECRET_SCALAR, KIND_PUBLIC_POINT, KIND_SECRET_POINT = 0, 1, 2, 3
+AFX_ERR_SHAPE = -5
 
 
 class PresentationBatch:
@@ -287,20 +288,23 @@ class Issuer:
         """Batch CredentialIssuance::verify (issuer.rs:48-57)."""
         return self._run(self._b.L.afx_verify_issuances, batch, 3, 1, debug)
 
-    def issue_batch(self, batch: RequestBatch, debug=False, out=None):
+    def issue_batch(self, batch: RequestBatch, debug=False, out=None, batchable=False):
         """Batch Issuer::issue (issuer.rs:111-124).  Returns (IssuanceBatch, status): the issuances in the layout
         verify_issuance_batch takes (attribute[n], t, U, V, challenge, responses[n+5]); status 0 = Ok, 1 = malformed request.
         out: optional preallocated uint8 [2n + 9][count][32] array for the result, e.g. from Issuer.host_array -- in page-locked
-        memory the device-to-host copy of (n + 9) x 32 bytes per item runs at the bus rate instead of through the driver's staging."""
+        memory the device-to-host copy of (n + 9) x 32 bytes per item runs at the bus rate instead of through the driver's staging.
+        batchable: the proofs as zkp's prove_batchable returns them, the challenge replaced by the commitments C_W, I, V -- the
+        [2n + 11][count][32] layout verify_issuance_batchable and verify_batchable_rlc(issuance=True) take."""
         n, count = len(batch.kinds), batch.count
         if batch.fields.shape[0] != 3 * n + 14:
             raise ValueError("a request batch has 3n + 14 fields")
         ptrs, keep = B._as_fields(batch.fields)
         cb = B.afx_presentation_batch(n, batch.kinds, count, ctypes.cast(ptrs, ctypes.POINTER(ctypes.c_void_p)), len(keep))
+        nw = 2 * n + (11 if batchable else 9)
         if out is None:
-            out = np.zeros((2 * n + 9, count, 32), np.uint8)
-        elif out.shape != (2 * n + 9, count, 32) or out.dtype != np.uint8 or not out.flags.c_contiguous:
-            raise ValueError("out must be a contiguous uint8 [2n + 9][count][32] array")
+            out = np.zeros((nw, count, 32), np.uint8)
+        elif out.shape != (nw, count, 32) or out.dtype != np.uint8 or not out.flags.c_contiguous:
+            raise ValueError("out must be a contiguous uint8 [%s][count][32] array" % ("2n + 11" if batchable else "2n + 9"))
         out[:n] = batch.fields[:n]
         optrs, okeep = B._as_fields(out[n:])
         ob = B.afx_issuance_out(ctypes.cast(optrs, ctypes.POINTER(ctypes.c_void_p)), len(okeep))
@@ -309,18 +313,24 @@ class Issuer:
         if debug:
             dump = {"commitments": np.zeros((3, count, 32), np.uint8), "status": np.zeros(count, np.uint32)}
             dbg = B.afx_debug_dump(None, dump["commitments"].ctypes.data, None, dump["status"].ctypes.data)
-        self._b.check(self._b.L.afx_issue(self._h, ctypes.byref(cb), ctypes.byref(ob), status.ctypes.data, ctypes.byref(dbg) if dbg is not None else None))
+        fn = self._b.L.afx_issue_batchable if batchable else self._b.L.afx_issue
+        self._b.check(fn(self._h, ctypes.byref(cb), ctypes.byref(ob), status.ctypes.data, ctypes.byref(dbg) if dbg is not None else None))
         for i, a in enumerate(okeep):            # _as_fields may have copied non-contiguous rows
             if a is not out[n + i] and not np.shares_memory(a, out):
                 out[n + i] = a
         res = IssuanceBatch(batch.kinds, out)
         return (res, status, dump) if debug else (res, status)
 
-    def show_batch(self, kinds, fields, debug=False, linked=False):
+    def show_batch(self, kinds, fields, debug=False, linked=False, batchable=False):
         """Batch AnonymousCredential::show (credential.rs:37-46).  kinds: the presentation's attribute kinds; fields: uint8
         [afx_show_num_fields][count][32] in the order documented in include/aeonflux_b200.h (credential, attributes, keypair,
-        rng bytes).  Returns (PresentationBatch, status) -- the batch can be passed to verify_batch as is."""
+        rng bytes).  Returns (PresentationBatch, status) -- the batch can be passed to verify_batch as is.  batchable: the proofs
+        as zkp's prove_batchable returns them (every challenge replaced by that proof's commitments), the layout verify_batchable
+        and verify_batchable_rlc take.  There is no linked BatchableProof statement: linked and batchable together raise
+        AFX_ERR_SHAPE."""
         kinds = bytes(kinds)
+        if linked and batchable:
+            self._b.check(AFX_ERR_SHAPE)
         fields = np.ascontiguousarray(fields, dtype=np.uint8)
         nf = self._b.L.afx_show_num_fields(len(kinds), kinds)
         if fields.ndim != 3 or fields.shape[0] != nf or fields.shape[2] != 32:
@@ -328,7 +338,8 @@ class Issuer:
         count = fields.shape[1]
         ptrs, keep = B._as_fields(fields)
         cb = B.afx_presentation_batch(len(kinds), kinds, count, ctypes.cast(ptrs, ctypes.POINTER(ctypes.c_void_p)), len(keep))
-        out = np.zeros((self.num_fields(kinds), count, 32), np.uint8)
+        nw = self._b.L.afx_batchable_num_fields(len(kinds), kinds) if batchable else self.num_fields(kinds)
+        out = np.zeros((nw, count, 32), np.uint8)
         optrs, okeep = B._as_fields(out)
         ob = B.afx_issuance_out(ctypes.cast(optrs, ctypes.POINTER(ctypes.c_void_p)), len(okeep))
         status = np.zeros(count, np.uint8)
@@ -337,7 +348,7 @@ class Issuer:
             ncm = self._b.L.afx_presentation_linked_num_commitments(len(kinds), kinds) if linked else self.num_commitments(kinds)
             dump = {"commitments": np.zeros((ncm, count, 32), np.uint8), "status": np.zeros(count, np.uint32)}
             dbg = B.afx_debug_dump(None, dump["commitments"].ctypes.data, None, dump["status"].ctypes.data)
-        fn = self._b.L.afx_show_linked if linked else self._b.L.afx_show
+        fn = self._b.L.afx_show_linked if linked else self._b.L.afx_show_batchable if batchable else self._b.L.afx_show
         self._b.check(fn(self._h, ctypes.byref(cb), ctypes.byref(ob), status.ctypes.data, ctypes.byref(dbg) if dbg is not None else None))
         res = PresentationBatch(kinds, out)
         return (res, status, dump) if debug else (res, status)
@@ -375,11 +386,17 @@ class Issuer:
         self._b.check(fn(self._h, len(kinds), kinds, count, inputs.ctypes.data, out.ctypes.data, status.ctypes.data))
         return out, status
 
-    def show_batch_device(self, kinds, count, fields_dev_ptr, out_dev_ptr, status_dev_ptr, stream=0):
-        self._b.check(self._b.L.afx_show_device(self._h, len(kinds), bytes(kinds), count, fields_dev_ptr, out_dev_ptr, status_dev_ptr, stream))
+    def show_batch_device(self, kinds, count, fields_dev_ptr, out_dev_ptr, status_dev_ptr, stream=0, batchable=False):
+        """Enqueue show_batch on device memory: out [n_out][count][32] with n_out = num_fields(kinds), or with batchable=True
+        afx_batchable_num_fields(kinds); count <= max_batch, no synchronisation."""
+        fn = self._b.L.afx_show_batchable_device if batchable else self._b.L.afx_show_device
+        self._b.check(fn(self._h, len(kinds), bytes(kinds), count, fields_dev_ptr, out_dev_ptr, status_dev_ptr, stream))
 
-    def issue_batch_device(self, kinds, count, fields_dev_ptr, out_dev_ptr, status_dev_ptr, stream=0):
-        self._b.check(self._b.L.afx_issue_device(self._h, len(kinds), bytes(kinds), count, fields_dev_ptr, out_dev_ptr, status_dev_ptr, stream))
+    def issue_batch_device(self, kinds, count, fields_dev_ptr, out_dev_ptr, status_dev_ptr, stream=0, batchable=False):
+        """Enqueue issue_batch on device memory: out [n + 9][count][32], or with batchable=True [n + 11][count][32] (t, U, V, the
+        commitments C_W, I, V, responses[n + 5]); count <= max_batch, no synchronisation."""
+        fn = self._b.L.afx_issue_batchable_device if batchable else self._b.L.afx_issue_device
+        self._b.check(fn(self._h, len(kinds), bytes(kinds), count, fields_dev_ptr, out_dev_ptr, status_dev_ptr, stream))
 
     def verify_issuance_batch_device(self, kinds, count, fields_dev_ptr, verdicts_dev_ptr, stream=0):
         self._b.check(self._b.L.afx_verify_issuances_device(self._h, len(kinds), bytes(kinds), count, fields_dev_ptr, verdicts_dev_ptr, stream))

@@ -243,6 +243,26 @@ int afx_show_device(afx_ctx* ctx, uint16_t n_attrs, const uint8_t* kinds, size_t
 int afx_show_wire(afx_ctx* ctx, uint16_t n_attrs, const uint8_t* kinds, size_t count, const uint8_t* inputs, uint8_t* presentations,
                   uint8_t* status);
 
+/* Issue and show in BatchableProof form: zkp 0.7's prove_batchable instead of prove_compact.  The prover is the same (same inputs,
+ * blindings, commitments and transcripts, hence the same challenges and responses); only its return value differs: the blinding
+ * commitments in place of each challenge.  The outputs are exactly what the BatchableProof verifiers above take:
+ *   afx_issue_batchable: output fields t, U, V, commitments[3] (constraint order C_W, I, V), responses[n + 5], i.e. n + 11 fields,
+ *       which with the request's attribute[n] in front is the afx_issuance_batchable_num_fields(n) = 2n + 11 layout of
+ *       afx_verify_issuances_batchable{,_rlc}.  Needs the issuer secret, like afx_issue.
+ *   afx_show_batchable: output fields in the afx_batchable_num_fields(n, kinds) layout of afx_verify_presentations_batchable{,_rlc}
+ *       (the main proof's challenge replaced by its commitments Z, C_x_1, then the C_y constraints; each proof of encryption's by
+ *       pk, C_y_1-E2, C_y_2', E1, C_y_3).  Needs no issuer secret, like afx_show.
+ * Inputs, status, chunking beyond max_batch, dbg and the *_device forms (count <= max_batch, out_dev = [n_out][count][32]) are those
+ * of afx_issue / afx_show.  A commitment that is the identity (possible only when blindings are zero) is written as its encoding,
+ * 32 zero bytes, with status 0: zkp's prover appends commitments without validating them.  zkp's verify_batchable, and the
+ * afx_verify_*_batchable calls, reject such a proof.  There is no linked BatchableProof statement. */
+int afx_issue_batchable(afx_ctx* ctx, const afx_request_batch* batch, const afx_issuance_out* out, uint8_t* status, afx_debug_dump* dbg);
+int afx_issue_batchable_device(afx_ctx* ctx, uint16_t n_attrs, const uint8_t* kinds, size_t count, const void* fields_dev, void* out_dev,
+                               void* status_dev, void* stream);
+int afx_show_batchable(afx_ctx* ctx, const afx_show_batch* batch, const afx_presentation_out* out, uint8_t* status, afx_debug_dump* dbg);
+int afx_show_batchable_device(afx_ctx* ctx, uint16_t n_attrs, const uint8_t* kinds, size_t count, const void* fields_dev, void* out_dev,
+                              void* status_dev, void* stream);
+
 /* Symmetric encryption of attributes: Plaintext::from(&[u8; 30]) (src/symmetric.rs:135-143 -> src/encoding.rs:56-70),
  * Keypair::encrypt (src/symmetric.rs:252-261) and Keypair::decrypt (src/symmetric.rs:273-289), in batch form.  User-side and
  * key-holder operations: they need no issuer secret (a context created with secret = NULL suffices) and do not use the system

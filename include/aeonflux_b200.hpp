@@ -13,6 +13,7 @@
 //   Issuer::issue(&self, CredentialRequest, &mut rng)                  Issuer::issue_batch(RequestBatch)          :111-124
 //   CredentialIssuance::verify(self, &sysparams, &issuer_params)       CredentialIssuance::verify_batch(Issuer&, IssuanceBatch)  :48-57
 //   AnonymousCredential::show(...)                                     Issuer::show_batch(ShowBatch)  (user side, no secret key)
+//   (zkp prove_batchable instead of prove_compact)                     issue_batch / show_batch with batchable = true
 //
 // A batch is one attribute shape (the kinds vector) and struct-of-arrays fields, each `count` x 32 bytes; the field orders are
 // documented in aeonflux_b200.h.  Structural mistakes (wrong field count, wrong attribute count) throw std::invalid_argument /
@@ -151,39 +152,43 @@ public:
         return to_results(v);
     }
     // Batch Issuer::issue.  Err(MacCreation) for the whole batch when the attribute count is not the issuer's (src/amacs.rs:285-287);
-    // otherwise the issuances (in IssuanceBatch layout) and a per-item Result.
-    std::pair<IssuanceBatch, std::vector<Result<>>> issue_batch(const RequestBatch& r) const {
-        size_t n = r.kinds.size(), count = r.count();
+    // otherwise the issuances (in IssuanceBatch layout) and a per-item Result.  batchable: zkp's prove_batchable form, the
+    // challenge replaced by the commitments C_W, I, V (2n + 11 fields, what afx_verify_issuances_batchable takes).
+    std::pair<IssuanceBatch, std::vector<Result<>>> issue_batch(const RequestBatch& r, bool batchable = false) const {
+        size_t n = r.kinds.size(), count = r.count(), nw = 2 * n + (batchable ? 11 : 9);
         IssuanceBatch out; out.kinds = r.kinds;
         if (n != number_of_attributes()) return {out, std::vector<Result<>>(count, Result<>::Err(CredentialError::MacCreation))};
         if (r.fields.size() != afx_request_num_fields((uint16_t)n)) throw std::invalid_argument("wrong number of request fields");
-        out.fields.assign(2 * n + 9, std::vector<uint8_t>(count * 32));
+        out.fields.assign(nw, std::vector<uint8_t>(count * 32));
         for (size_t i = 0; i < n; i++) out.fields[i] = r.fields[i];
         auto in = r.pointers();
         std::vector<uint8_t*> op;
-        for (size_t w = n; w < 2 * n + 9; w++) op.push_back(out.fields[w].data());
+        for (size_t w = n; w < nw; w++) op.push_back(out.fields[w].data());
         afx_request_batch b{(uint16_t)n, r.kinds.data(), count, in.data(), in.size()};
         afx_issuance_out o{op.data(), op.size()};
         std::vector<uint8_t> st(count);
-        int rc = afx_issue(ctx_, &b, &o, st.data(), nullptr);
+        int rc = batchable ? afx_issue_batchable(ctx_, &b, &o, st.data(), nullptr) : afx_issue(ctx_, &b, &o, st.data(), nullptr);
         if (rc != AFX_OK) throw Error(rc);
         std::vector<Result<>> res;
         for (uint8_t s : st) res.push_back(s == 0 ? Result<>::Ok() : Result<>::Err(CredentialError::BadAttribute));
         return {out, res};
     }
-    // Batch AnonymousCredential::show (user side; works on a context without the secret key)
-    std::pair<PresentationBatch, std::vector<Result<>>> show_batch(const ShowBatch& s) const {
+    // Batch AnonymousCredential::show (user side; works on a context without the secret key).  batchable: zkp's prove_batchable
+    // form, every challenge replaced by that proof's commitments (what verify_batchable takes).
+    std::pair<PresentationBatch, std::vector<Result<>>> show_batch(const ShowBatch& s, bool batchable = false) const {
         size_t count = s.count();
         if (s.fields.size() != afx_show_num_fields((uint16_t)s.kinds.size(), s.kinds.data())) throw std::invalid_argument("wrong number of show fields");
         PresentationBatch out; out.kinds = s.kinds;
-        out.fields.assign(afx_presentation_num_fields((uint16_t)s.kinds.size(), s.kinds.data()), std::vector<uint8_t>(count * 32));
+        size_t nw = batchable ? afx_batchable_num_fields((uint16_t)s.kinds.size(), s.kinds.data())
+                              : afx_presentation_num_fields((uint16_t)s.kinds.size(), s.kinds.data());
+        out.fields.assign(nw, std::vector<uint8_t>(count * 32));
         auto in = s.pointers();
         std::vector<uint8_t*> op;
         for (auto& f : out.fields) op.push_back(f.data());
         afx_show_batch b{(uint16_t)s.kinds.size(), s.kinds.data(), count, in.data(), in.size()};
         afx_presentation_out o{op.data(), op.size()};
         std::vector<uint8_t> st(count);
-        int rc = afx_show(ctx_, &b, &o, st.data(), nullptr);
+        int rc = batchable ? afx_show_batchable(ctx_, &b, &o, st.data(), nullptr) : afx_show(ctx_, &b, &o, st.data(), nullptr);
         if (rc != AFX_OK) throw Error(rc);
         std::vector<Result<>> res;
         for (uint8_t x : st) res.push_back(x == 0 ? Result<>::Ok() : Result<>::Err(CredentialError::BadAttribute));
