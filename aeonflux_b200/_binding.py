@@ -39,7 +39,8 @@ class Binding:
                "afx_verify_presentations_linked_wire", "afx_show_linked", "afx_show_linked_wire", "afx_issuance_batchable_num_fields", "afx_verify_issuances_batchable", "afx_verify_issuances_batchable_rlc", "afx_get_rlc_stats",
                "afx_encode_plaintexts", "afx_encrypt", "afx_decrypt", "afx_encode_plaintexts_device", "afx_encrypt_device",
                "afx_decrypt_device", "afx_derive_keypairs", "afx_derive_keypairs_device", "afx_issue_batchable", "afx_issue_batchable_device",
-               "afx_show_batchable", "afx_show_batchable_device"]
+               "afx_show_batchable", "afx_show_batchable_device", "afx_verify_presentations_mixed_wire", "afx_verify_issuances_mixed_wire",
+               "afx_multi_verify_presentations_mixed_wire", "afx_multi_verify_issuances_mixed_wire"]
 
     def __init__(self, cdll):
         L = self.L = cdll
@@ -170,6 +171,10 @@ class Binding:
         for f in ("afx_multi_verify_presentations_wire", "afx_multi_verify_issuances_wire"):
             getattr(L, f).restype = ctypes.c_int
             getattr(L, f).argtypes = [vp, ctypes.c_uint16, ctypes.c_char_p, sz, vp, vp]
+        for f in ("afx_verify_presentations_mixed_wire", "afx_verify_issuances_mixed_wire", "afx_multi_verify_presentations_mixed_wire",
+                  "afx_multi_verify_issuances_mixed_wire"):
+            getattr(L, f).restype = ctypes.c_int
+            getattr(L, f).argtypes = [vp, ctypes.c_uint16, ctypes.c_char_p, sz, sz, vp, vp, vp]
         L.afx_multi_issue.restype = ctypes.c_int
         L.afx_multi_issue.argtypes = [vp, ctypes.POINTER(afx_presentation_batch), ctypes.POINTER(afx_issuance_out), vp]
 
@@ -196,3 +201,21 @@ def _as_fields(fields):
     arrs = [np.ascontiguousarray(f, dtype=np.uint8) for f in fields]
     ptrs = (ctypes.c_void_p * len(arrs))(*[a.ctypes.data for a in arrs])
     return ptrs, arrs
+
+
+def verify_mixed_wire(binding, fn, handle, shape_kinds, records, shape_ids, issuance):
+    """Marshals afx_[multi_]verify_{presentations,issuances}_mixed_wire: shape_kinds = the kind vectors of the call, records = uint8
+    array holding the records concatenated in order (record i in the wire layout of shape shape_ids[i]), shape_ids = uint8 [count]."""
+    shape_kinds = [bytes(k) for k in shape_kinds]
+    n = len(shape_kinds[0]) if shape_kinds else 0
+    if any(len(k) != n for k in shape_kinds):
+        raise ValueError("every kind vector of a call has the issuer's attribute count")
+    records = np.ascontiguousarray(records, dtype=np.uint8).reshape(-1)
+    ids = np.ascontiguousarray(shape_ids, dtype=np.uint8).reshape(-1)
+    if len(ids) and int(ids.max()) < len(shape_kinds):      # an unknown shape id is the library's error to report
+        sizes = np.array([32 * ((2 * n + 9) if issuance else binding.L.afx_presentation_num_fields(n, k)) for k in shape_kinds], np.int64)
+        if int(sizes[ids].sum()) != records.size:
+            raise ValueError("records must hold exactly one record of its shape per shape id")
+    verdicts = np.zeros(len(ids), np.uint8)
+    binding.check(fn(handle, n, b"".join(shape_kinds), len(shape_kinds), len(ids), records.ctypes.data, ids.ctypes.data, verdicts.ctypes.data))
+    return verdicts

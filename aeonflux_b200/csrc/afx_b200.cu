@@ -278,6 +278,25 @@ __global__ void __launch_bounds__(256) k_verdict(Workspace ws, uint8_t* verdicts
     if (item < ws.count) verdicts[item] = ws.status[item] != 0;
 }
 
+// Mixed-shape calls: one CTA per tile of BUCKET_TILE records.  Every thread locates one record (engine.cuh:bucket_locate, over the
+// tile's ids in shared memory); then each warp copies whole records, its lanes on consecutive 16-byte quads of one record.
+__global__ void __launch_bounds__(BUCKET_TILE) k_bucket_records(BucketArgs a) {
+    __shared__ uint8_t ids[BUCKET_TILE];
+    __shared__ u32 rec_words[256];
+    __shared__ u64 src[BUCKET_TILE], dst[BUCKET_TILE];
+    const u32 i0 = blockIdx.x * BUCKET_TILE, n = a.count - i0 < BUCKET_TILE ? a.count - i0 : BUCKET_TILE, t = threadIdx.x;
+    if (t < n) ids[t] = a.ids[i0 + t];
+    if (t < a.n_shapes) rec_words[t] = a.rec_words[t];
+    __syncthreads();
+    if (t < n) a.slot[i0 + t] = bucket_locate(a, ids, rec_words, i0 + t, src[t], dst[t]);
+    __syncthreads();
+    for (u32 r = t / 32; r < n; r += BUCKET_TILE / 32) bucket_copy(a.records + src[r], a.fields + dst[r], rec_words[ids[r]], t % 32, 32);
+}
+__global__ void __launch_bounds__(256) k_scatter_verdicts(const uint8_t* bucket_verdicts, const u32* slot, uint8_t* verdicts, u32 count) {
+    u32 i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < count) scatter_verdict_job(bucket_verdicts, slot, verdicts, i);
+}
+
 // per-issuer setup: one thread per (constant point, multiple)
 __global__ void __launch_bounds__(128) k_ctab_setup(const u32* enc, u32 ncp, u32* ctabs, u32* encneg, u32* bad, u32 entries, int bits) {
     u32 t = blockIdx.x * blockDim.x + threadIdx.x;
@@ -531,6 +550,10 @@ static u32 be_launch_rlc(const Workspace& ws, const RlcDesc* d_desc, u32 ncterms
 }
 static void be_launch_verdict(const Workspace& ws, uint8_t* verdicts, be_stream s) {
     k_verdict<<<grid_for(ws.count, 256, 1), 256, 0, s>>>(ws, verdicts);
+}
+static void be_launch_bucket_records(const BucketArgs& a, be_stream s) { k_bucket_records<<<grid_for(a.count, BUCKET_TILE, 1), BUCKET_TILE, 0, s>>>(a); }
+static void be_launch_scatter_verdicts(const uint8_t* bucket_verdicts, const u32* slot, uint8_t* verdicts, u32 count, be_stream s) {
+    k_scatter_verdicts<<<grid_for(count, 256, 1), 256, 0, s>>>(bucket_verdicts, slot, verdicts, count);
 }
 // entries = 2^bits multiples 1..2^bits of every constant point
 static void be_launch_ctab_setup(const u32* d_enc, u32 ncp, u32* d_ctabs, u32* d_encneg, u32* d_bad, int bits, be_stream s) {

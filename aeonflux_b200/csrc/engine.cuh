@@ -1204,4 +1204,51 @@ AFX_HD void keypair_scalars_job(const u32* ms, u32* rows, u32 count, u32 item) {
     }
 }
 
+// ---- mixed-shape verify calls: device-side bucketing of a pass of records of several shapes ------------------------------------
+// A pass is `count` consecutive records as the caller concatenated them, record i being rec_words[ids[i]] words long.  Each shape's
+// records are copied into its own item-major bucket (the *_wire layout), in record order, so that the shape's verify program runs on
+// the bucket as it is.  The host scans the ids anyway (to validate them and count each shape); it records the running counts and
+// the running word offset every BUCKET_TILE records, which leaves the device a rank and an offset within one tile per record.
+constexpr u32 BUCKET_TILE = 256;
+struct BucketArgs {
+    const u32* records;      // the pass's records as received
+    u32* fields;             // the buckets: shape s's bucket starts at word base_word[s]
+    const uint8_t* ids;      // [count] shape id of every record
+    const u32* rec_words;    // [n_shapes] record length in words (n_fields * 8)
+    const u64* base_word;    // [n_shapes]
+    const u32* vbase;        // [n_shapes] first index of shape s's bucket in the bucket-order verdict array
+    const u32* tile_rank;    // [tiles][n_shapes] records of shape s in the pass before the tile
+    const u64* tile_src;     // [tiles] word offset of the tile's first record in `records`
+    u32* slot;               // [count] out: the record's index in the bucket-order verdict array
+    u32 count, n_shapes;
+};
+
+// Record i: its index in the bucket-order verdict array, its word offset in the pass (src) and in the buckets (dst).  The rank
+// within its shape counts the earlier records of the tile with the same id, so the bucket keeps the record order.  tile_ids are
+// the ids of i's tile, rec_words the record lengths (the kernel passes its shared-memory copies).
+AFX_HD u32 bucket_locate(const BucketArgs& a, const uint8_t* tile_ids, const u32* rec_words, u32 i, u64& src, u64& dst) {
+    const u32 t = i / BUCKET_TILE, j_end = i % BUCKET_TILE, s = tile_ids[j_end];
+    u32 rank = a.tile_rank[(size_t)t * a.n_shapes + s];
+    u64 off = a.tile_src[t];
+    for (u32 j = 0; j < j_end; j++) {
+        const u32 sj = tile_ids[j];
+        rank += sj == s;
+        off += rec_words[sj];
+    }
+    src = off;
+    dst = a.base_word[s] + (u64)rank * rec_words[s];
+    return a.vbase[s] + rank;
+}
+
+// Copy one record's words in 16-byte quads, lane `lane` of `nlanes` taking every nlanes-th quad (a warp moves 512 contiguous bytes per step).
+AFX_HD void bucket_copy(const u32* src, u32* dst, u32 words, u32 lane, u32 nlanes) {
+    u32 q[4];
+    for (u32 k = 4 * lane; k < words; k += 4 * nlanes) { load4(q, src + k); store4(dst + k, q); }
+}
+
+// Verdict of record i, read from its bucket's verdict array.
+AFX_HD void scatter_verdict_job(const uint8_t* bucket_verdicts, const u32* slot, uint8_t* verdicts, u32 i) {
+    verdicts[i] = bucket_verdicts[slot[i]];
+}
+
 }  // namespace afx

@@ -284,6 +284,14 @@ class Issuer:
         self._b.check(fn(self._h, len(kinds), bytes(kinds), items.shape[0], items.ctypes.data, verdicts.ctypes.data))
         return verdicts
 
+    def verify_mixed_wire(self, shape_kinds, records, shape_ids, issuance=False):
+        """Batch Issuer::verify (or CredentialIssuance::verify) over wire records of several shapes of this issuer in one call:
+        shape_kinds = list of kind vectors, records = uint8 array of the records concatenated in order (record i is an item of
+        shape shape_ids[i] in the verify_wire layout), shape_ids = uint8 [count].  The records are bucketed by shape on the
+        device; verdicts come back in record order."""
+        fn = self._b.L.afx_verify_issuances_mixed_wire if issuance else self._b.L.afx_verify_presentations_mixed_wire
+        return B.verify_mixed_wire(self._b, fn, self._h, shape_kinds, records, shape_ids, issuance)
+
     def verify_issuance_batch(self, batch: IssuanceBatch, debug=False):
         """Batch CredentialIssuance::verify (issuer.rs:48-57)."""
         return self._run(self._b.L.afx_verify_issuances, batch, 3, 1, debug)

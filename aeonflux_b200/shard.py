@@ -197,6 +197,12 @@ class MultiGpuIssuer:
         self._b.check(fn(self._h, len(kinds), kinds, items.shape[0], items.ctypes.data, verdicts.ctypes.data))
         return verdicts
 
+    def verify_mixed_wire(self, shape_kinds, records, shape_ids, issuance=False) -> np.ndarray:
+        """Issuer.verify_mixed_wire across the devices: device k takes records [k*N/G, (k+1)*N/G) and buckets them itself."""
+        from . import _binding as B
+        fn = self._b.L.afx_multi_verify_issuances_mixed_wire if issuance else self._b.L.afx_multi_verify_presentations_mixed_wire
+        return B.verify_mixed_wire(self._b, fn, self._h, shape_kinds, records, shape_ids, issuance)
+
     def issue_batch(self, batch):
         """Batch Issuer::issue across the devices (request layout of Issuer.issue_batch) -> (IssuanceBatch, status)."""
         import ctypes

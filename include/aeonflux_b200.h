@@ -170,6 +170,28 @@ int afx_verify_presentations_wire(afx_ctx* ctx, uint16_t n_attrs, const uint8_t*
 int afx_verify_issuances_wire(afx_ctx* ctx, uint16_t n_attrs, const uint8_t* kinds, size_t count, const uint8_t* items,
                               uint8_t* verdicts);
 
+/* Wire records of SEVERAL shapes of the context's issuer in one call: the batch form of Issuer::verify over whatever presentations
+ * the issuer receives, each user having chosen which attributes to hide (src/credential.rs:53-97), or of CredentialIssuance::verify
+ * over issuances of several request kinds.
+ *   shape_kinds = [n_shapes][n_attrs] the kind vectors of the call, 1 <= n_shapes <= 255 (a vector may be listed twice)
+ *   shape_ids   = [count] shape of each record, < n_shapes
+ *   records     = the records concatenated in order, record i being its shape's item in the *_wire layout above:
+ *                 afx_presentation_num_fields(n_attrs, kinds) * 32 bytes, or (2 * n_attrs + 9) * 32 bytes for an issuance
+ * verdicts[i] is what afx_verify_{presentations,issuances}_wire gives record i alone under its shape.  Checked before any device work
+ * and before anything is written to verdicts: AFX_ERR_ARG for n_shapes out of range, a shape id >= n_shapes, a null pointer with
+ * count > 0 (shape_kinds: always) or submissions outstanding; AFX_ERR_SHAPE for a kind vector the issuer cannot verify;
+ * AFX_ERR_NO_SECRET for presentations on a context without the issuer secret.  count = 0 is AFX_OK.
+ * The call works in passes of at most max_batch consecutive records of any mix.  Each pass's bytes are copied to the device once,
+ * as received (the copy of pass i + 1 under the kernels of pass i); a kernel copies every record into the item-major bucket of its
+ * shape, keeping the record order, the verify program of each shape present runs over its bucket, and the verdicts are put back in
+ * record order before one copy to the host.  The host reads only the shape ids.  Device memory: the workspace of the largest shape
+ * of the call at max_batch items, plus three [max_batch][largest record] buffers (the pass as received, twice, and the buckets),
+ * plus about 2 * (6 + 4 * n_shapes / 256) bytes of bucketing arrays per record of max_batch. */
+int afx_verify_presentations_mixed_wire(afx_ctx* ctx, uint16_t n_attrs, const uint8_t* shape_kinds, size_t n_shapes, size_t count,
+                                        const uint8_t* records, const uint8_t* shape_ids, uint8_t* verdicts);
+int afx_verify_issuances_mixed_wire(afx_ctx* ctx, uint16_t n_attrs, const uint8_t* shape_kinds, size_t n_shapes, size_t count,
+                                    const uint8_t* records, const uint8_t* shape_ids, uint8_t* verdicts);
+
 /* Same as afx_verify_issuances with the batch resident on the device ([2*n_attrs + 9][count][32] contiguous). */
 int afx_verify_issuances_device(afx_ctx* ctx, uint16_t n_attrs, const uint8_t* kinds, size_t count, const void* fields_dev,
                                 void* verdicts_dev, void* stream);
@@ -352,6 +374,11 @@ int afx_multi_verify_presentations_wire(afx_multi* m, uint16_t n_attrs, const ui
 int afx_multi_verify_issuances(afx_multi* m, const afx_issuance_batch* batch, uint8_t* verdicts);
 int afx_multi_verify_issuances_wire(afx_multi* m, uint16_t n_attrs, const uint8_t* kinds, size_t count, const uint8_t* items,
                                     uint8_t* verdicts);
+/* The mixed-shape calls across the devices: contiguous record slices as above, each device bucketing its own slice. */
+int afx_multi_verify_presentations_mixed_wire(afx_multi* m, uint16_t n_attrs, const uint8_t* shape_kinds, size_t n_shapes, size_t count,
+                                              const uint8_t* records, const uint8_t* shape_ids, uint8_t* verdicts);
+int afx_multi_verify_issuances_mixed_wire(afx_multi* m, uint16_t n_attrs, const uint8_t* shape_kinds, size_t n_shapes, size_t count,
+                                          const uint8_t* records, const uint8_t* shape_ids, uint8_t* verdicts);
 int afx_multi_issue(afx_multi* m, const afx_request_batch* batch, const afx_issuance_out* out, uint8_t* status);
 
 /* Streamed verification of MIXED shapes (BASELINE configs[4]; SURVEY 8d config 5: "bucketed by shape into chunks").  A stream is a

@@ -151,6 +151,21 @@ public:
         if (rc != AFX_OK) throw Error(rc);
         return to_results(v);
     }
+    // ... over presentations of any of `shape_kinds` (each user hides what it chooses): records = the wire records concatenated in
+    // order, record i of shape shape_ids[i]; bucketed by shape on the device, results in record order
+    std::vector<Result<>> verify_batch(const std::vector<std::vector<uint8_t>>& shape_kinds, const uint8_t* records,
+                                       const std::vector<uint8_t>& shape_ids) const {
+        std::vector<uint8_t> flat;
+        for (const auto& k : shape_kinds) {
+            if (k.size() != shape_kinds[0].size()) throw std::invalid_argument("every kind vector has the issuer's attribute count");
+            flat.insert(flat.end(), k.begin(), k.end());
+        }
+        const uint16_t n = shape_kinds.empty() ? 0 : (uint16_t)shape_kinds[0].size();
+        std::vector<uint8_t> v(shape_ids.size());
+        int rc = afx_verify_presentations_mixed_wire(ctx_, n, flat.data(), shape_kinds.size(), shape_ids.size(), records, shape_ids.data(), v.data());
+        if (rc != AFX_OK) throw Error(rc);
+        return to_results(v);
+    }
     // Batch Issuer::issue.  Err(MacCreation) for the whole batch when the attribute count is not the issuer's (src/amacs.rs:285-287);
     // otherwise the issuances (in IssuanceBatch layout) and a per-item Result.  batchable: zkp's prove_batchable form, the
     // challenge replaced by the commitments C_W, I, V (2n + 11 fields, what afx_verify_issuances_batchable takes).

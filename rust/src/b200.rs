@@ -138,6 +138,17 @@ impl B200Context {
         Ok(verdicts)
     }
 
+    /// Batch `Issuer::verify` (issuance: `CredentialIssuance::verify`) over wire records of several shapes of this issuer:
+    /// `records` = the records concatenated in order, record i of shape `shape_kinds[shape_ids[i]]`; bucketed on the device.
+    pub fn verify_mixed_wire(&self, issuance: bool, shape_kinds: &[&[u8]], records: &[u8], shape_ids: &[u8]) -> Result<Vec<u8>, B200Error> {
+        let (n, flat) = mixed_shapes(issuance, shape_kinds, records, shape_ids)?;
+        let mut verdicts = vec![0u8; shape_ids.len()];
+        let f = if issuance { afx_verify_issuances_mixed_wire } else { afx_verify_presentations_mixed_wire };
+        let rc = unsafe { f(self.ctx, n, flat.as_ptr(), shape_kinds.len(), shape_ids.len(), records.as_ptr(), shape_ids.as_ptr(), verdicts.as_mut_ptr()) };
+        if rc != 0 { return Err(B200Error(rc)); }
+        Ok(verdicts)
+    }
+
     /// Batch `CredentialIssuance::verify` over struct-of-arrays fields (`attribute[n], t, U, V, challenge, responses[n+5]`).
     pub fn verify_issuances(&self, kinds: &[u8], fields: &[&[u8]]) -> Result<Vec<u8>, B200Error> {
         let n_fields = 2 * kinds.len() + 9;
@@ -189,6 +200,19 @@ impl Drop for B200Context {
 }
 
 
+/// The kind vectors of a mixed-shape call, flattened, after checking that `records` holds exactly one record per shape id (the
+/// library takes no length and reads the records the shape ids describe).
+fn mixed_shapes(issuance: bool, shape_kinds: &[&[u8]], records: &[u8], shape_ids: &[u8]) -> Result<(u16, Vec<u8>), B200Error> {
+    let n = shape_kinds.first().map_or(0, |k| k.len());
+    if shape_kinds.iter().any(|k| k.len() != n) { return Err(B200Error(-1)); }
+    let bytes: Vec<usize> = shape_kinds.iter()
+        .map(|k| 32 * if issuance { 2 * n + 9 } else { unsafe { afx_presentation_num_fields(n as u16, k.as_ptr()) } }).collect();
+    let mut total = 0usize;
+    for &s in shape_ids { match bytes.get(s as usize) { Some(b) => total += b, None => return Err(B200Error(-1)) } }
+    if total != records.len() { return Err(B200Error(-1)); }
+    Ok((n as u16, shape_kinds.concat()))
+}
+
 /// Several B200s behind one handle (`afx_multi_*`): the library replicates the issuer context on every listed device, keeps one
 /// host thread per device, cuts a batch into contiguous item slices (device k of G takes `[k*N/G, (k+1)*N/G)`) and lets every
 /// device write its slice of the verdict array.  This is what `Issuer::verify_batch` binds when the box has more than one GPU.
@@ -222,6 +246,16 @@ impl B200Multi {
         let rc = unsafe {
             afx_multi_verify_presentations_wire(self.m, kinds.len() as u16, kinds.as_ptr(), count, items.as_ptr(), verdicts.as_mut_ptr())
         };
+        if rc != 0 { return Err(B200Error(rc)); }
+        Ok(verdicts)
+    }
+
+    /// `B200Context::verify_mixed_wire` sharded over the devices: each device buckets its own slice of records.
+    pub fn verify_mixed_wire(&self, issuance: bool, shape_kinds: &[&[u8]], records: &[u8], shape_ids: &[u8]) -> Result<Vec<u8>, B200Error> {
+        let (n, flat) = mixed_shapes(issuance, shape_kinds, records, shape_ids)?;
+        let mut verdicts = vec![0u8; shape_ids.len()];
+        let f = if issuance { afx_multi_verify_issuances_mixed_wire } else { afx_multi_verify_presentations_mixed_wire };
+        let rc = unsafe { f(self.m, n, flat.as_ptr(), shape_kinds.len(), shape_ids.len(), records.as_ptr(), shape_ids.as_ptr(), verdicts.as_mut_ptr()) };
         if rc != 0 { return Err(B200Error(rc)); }
         Ok(verdicts)
     }
