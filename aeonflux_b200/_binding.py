@@ -40,7 +40,8 @@ class Binding:
                "afx_encode_plaintexts", "afx_encrypt", "afx_decrypt", "afx_encode_plaintexts_device", "afx_encrypt_device",
                "afx_decrypt_device", "afx_derive_keypairs", "afx_derive_keypairs_device", "afx_issue_batchable", "afx_issue_batchable_device",
                "afx_show_batchable", "afx_show_batchable_device", "afx_verify_presentations_mixed_wire", "afx_verify_issuances_mixed_wire",
-               "afx_multi_verify_presentations_mixed_wire", "afx_multi_verify_issuances_mixed_wire"]
+               "afx_multi_verify_presentations_mixed_wire", "afx_multi_verify_issuances_mixed_wire", "afx_issue_mixed_wire",
+               "afx_show_mixed_wire", "afx_multi_issue_mixed_wire"]
 
     def __init__(self, cdll):
         L = self.L = cdll
@@ -175,6 +176,9 @@ class Binding:
                   "afx_multi_verify_issuances_mixed_wire"):
             getattr(L, f).restype = ctypes.c_int
             getattr(L, f).argtypes = [vp, ctypes.c_uint16, ctypes.c_char_p, sz, sz, vp, vp, vp]
+        for f in ("afx_issue_mixed_wire", "afx_show_mixed_wire", "afx_multi_issue_mixed_wire"):
+            getattr(L, f).restype = ctypes.c_int
+            getattr(L, f).argtypes = [vp, ctypes.c_uint16, ctypes.c_char_p, sz, sz, vp, vp, vp, vp]
         L.afx_multi_issue.restype = ctypes.c_int
         L.afx_multi_issue.argtypes = [vp, ctypes.POINTER(afx_presentation_batch), ctypes.POINTER(afx_issuance_out), vp]
 
@@ -219,3 +223,49 @@ def verify_mixed_wire(binding, fn, handle, shape_kinds, records, shape_ids, issu
     verdicts = np.zeros(len(ids), np.uint8)
     binding.check(fn(handle, n, b"".join(shape_kinds), len(shape_kinds), len(ids), records.ctypes.data, ids.ctypes.data, verdicts.ctypes.data))
     return verdicts
+
+
+def mixed_record_bytes(binding, shape_kinds, what):
+    """Record length in bytes of every kind vector of a mixed call: what = "request", "issuance", "show" (a show input) or
+    "presentation"."""
+    L = binding.L
+    size = {"request": lambda k: 3 * len(k) + 14, "issuance": lambda k: 2 * len(k) + 9,
+            "show": lambda k: L.afx_show_num_fields(len(k), k), "presentation": lambda k: L.afx_presentation_num_fields(len(k), k)}[what]
+    return np.array([32 * size(bytes(k)) for k in shape_kinds], np.int64)
+
+
+def record_offsets(sizes, shape_ids):
+    """Byte offsets [count + 1] of records concatenated in order, record i of sizes[shape_ids[i]] bytes: record i is
+    blob[offsets[i]:offsets[i + 1]]."""
+    ids = np.asarray(shape_ids, np.uint8).reshape(-1)
+    offsets = np.zeros(len(ids) + 1, np.int64)
+    np.cumsum(np.asarray(sizes, np.int64)[ids], out=offsets[1:])
+    return offsets
+
+
+def prove_mixed_wire(binding, fn, handle, shape_kinds, inputs, shape_ids, issue, out=None):
+    """Marshals afx_[multi_]{issue,show}_mixed_wire: shape_kinds = the kind vectors of the call, inputs = uint8 array holding the
+    requests (or show inputs) concatenated in order, record i of shape shape_ids[i], shape_ids = uint8 [count].  Returns (the
+    output records concatenated in order as a flat uint8 array, status).  out: optional preallocated (e.g. page-locked) contiguous
+    uint8 array of exactly the output size, returned flattened."""
+    shape_kinds = [bytes(k) for k in shape_kinds]
+    n = len(shape_kinds[0]) if shape_kinds else 0
+    if any(len(k) != n for k in shape_kinds):
+        raise ValueError("every kind vector of a call has the issuer's attribute count")
+    inputs = np.ascontiguousarray(inputs, dtype=np.uint8).reshape(-1)
+    ids = np.ascontiguousarray(shape_ids, dtype=np.uint8).reshape(-1)
+    out_bytes = 0
+    if len(ids) and int(ids.max()) < len(shape_kinds):      # an unknown shape id is the library's error to report
+        in_sizes = mixed_record_bytes(binding, shape_kinds, "request" if issue else "show")
+        if int(in_sizes[ids].sum()) != inputs.size:
+            raise ValueError("inputs must hold exactly one record of its shape per shape id")
+        out_bytes = int(mixed_record_bytes(binding, shape_kinds, "issuance" if issue else "presentation")[ids].sum())
+    if out is None:
+        out = np.zeros(out_bytes, np.uint8)
+    elif out.dtype != np.uint8 or not out.flags.c_contiguous or out.size != out_bytes:
+        raise ValueError("out must be a contiguous uint8 array of %d bytes" % out_bytes)
+    out = out.reshape(-1)
+    status = np.zeros(len(ids), np.uint8)
+    binding.check(fn(handle, n, b"".join(shape_kinds), len(shape_kinds), len(ids), inputs.ctypes.data, ids.ctypes.data, out.ctypes.data,
+                     status.ctypes.data))
+    return out, status

@@ -296,6 +296,20 @@ __global__ void __launch_bounds__(256) k_scatter_verdicts(const uint8_t* bucket_
     u32 i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i < count) scatter_verdict_job(bucket_verdicts, slot, verdicts, i);
 }
+// Mixed-shape prover calls, the inverse of k_bucket_records: every thread locates one record's output (engine.cuh:unbucket_locate)
+// and scatters its status byte; then each warp copies whole output records back into record order.
+__global__ void __launch_bounds__(BUCKET_TILE) k_unbucket_records(UnbucketArgs a) {
+    __shared__ uint8_t ids[BUCKET_TILE];
+    __shared__ u32 out_words[256];
+    __shared__ u64 src[BUCKET_TILE], dst[BUCKET_TILE];
+    const u32 i0 = blockIdx.x * BUCKET_TILE, n = a.count - i0 < BUCKET_TILE ? a.count - i0 : BUCKET_TILE, t = threadIdx.x;
+    if (t < n) ids[t] = a.ids[i0 + t];
+    if (t < a.n_shapes) out_words[t] = a.out_words[t];
+    __syncthreads();
+    if (t < n) a.status[i0 + t] = unbucket_locate(a, ids, out_words, i0 + t, src[t], dst[t]);
+    __syncthreads();
+    for (u32 r = t / 32; r < n; r += BUCKET_TILE / 32) bucket_copy(a.outputs + src[r], a.records + dst[r], out_words[ids[r]], t % 32, 32);
+}
 
 // per-issuer setup: one thread per (constant point, multiple)
 __global__ void __launch_bounds__(128) k_ctab_setup(const u32* enc, u32 ncp, u32* ctabs, u32* encneg, u32* bad, u32 entries, int bits) {
@@ -555,6 +569,7 @@ static void be_launch_bucket_records(const BucketArgs& a, be_stream s) { k_bucke
 static void be_launch_scatter_verdicts(const uint8_t* bucket_verdicts, const u32* slot, uint8_t* verdicts, u32 count, be_stream s) {
     k_scatter_verdicts<<<grid_for(count, 256, 1), 256, 0, s>>>(bucket_verdicts, slot, verdicts, count);
 }
+static void be_launch_unbucket_records(const UnbucketArgs& a, be_stream s) { k_unbucket_records<<<grid_for(a.count, BUCKET_TILE, 1), BUCKET_TILE, 0, s>>>(a); }
 // entries = 2^bits multiples 1..2^bits of every constant point
 static void be_launch_ctab_setup(const u32* d_enc, u32 ncp, u32* d_ctabs, u32* d_encneg, u32* d_bad, int bits, be_stream s) {
     u32 entries = 1u << bits, total = ncp * entries;

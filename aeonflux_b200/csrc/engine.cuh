@@ -1251,4 +1251,33 @@ AFX_HD void scatter_verdict_job(const uint8_t* bucket_verdicts, const u32* slot,
     verdicts[i] = bucket_verdicts[slot[i]];
 }
 
+// ---- mixed-shape prover calls: the inverse of the bucketing, for the prover outputs -------------------------------------------
+// Each shape's prover program writes its output records item-major into its own region (out_base[s]), in bucket order.  Every record
+// goes back to its position in the pass, and its status byte with it.  The rank comes from the slot k_bucket_records wrote; the host
+// records the running output word offset every BUCKET_TILE records, as it does for the inputs.
+struct UnbucketArgs {
+    const u32* outputs;             // the provers' output regions: shape s's starts at word out_base[s]
+    u32* records;                   // out: the pass's output records in record order
+    const uint8_t* ids;             // [count] shape id of every record
+    const u32* out_words;           // [n_shapes] output record length in words
+    const u64* out_base;            // [n_shapes]
+    const u32* vbase;               // [n_shapes] first index of shape s in the bucket-order status array
+    const u64* tile_dst;            // [tiles] word offset of the tile's first output record in `records`
+    const u32* slot;                // [count] the record's index in the bucket-order status array (k_bucket_records)
+    const uint8_t* bucket_status;   // [count] status in bucket order
+    uint8_t* status;                // [count] out: status in record order
+    u32 count, n_shapes;
+};
+
+// Record i: its status byte, its word offset in the output regions (src) and in the pass's output (dst).  tile_ids are the ids of
+// i's tile, out_words the output record lengths (the kernel passes its shared-memory copies).
+AFX_HD uint8_t unbucket_locate(const UnbucketArgs& a, const uint8_t* tile_ids, const u32* out_words, u32 i, u64& src, u64& dst) {
+    const u32 t = i / BUCKET_TILE, j_end = i % BUCKET_TILE, s = tile_ids[j_end], slot = a.slot[i];
+    u64 off = a.tile_dst[t];
+    for (u32 j = 0; j < j_end; j++) off += out_words[tile_ids[j]];
+    dst = off;
+    src = a.out_base[s] + (u64)(slot - a.vbase[s]) * out_words[s];
+    return a.bucket_status[slot];
+}
+
 }  // namespace afx

@@ -292,6 +292,27 @@ class Issuer:
         fn = self._b.L.afx_verify_issuances_mixed_wire if issuance else self._b.L.afx_verify_presentations_mixed_wire
         return B.verify_mixed_wire(self._b, fn, self._h, shape_kinds, records, shape_ids, issuance)
 
+    def issue_mixed_wire(self, shape_kinds, requests, shape_ids, out=None):
+        """Batch Issuer::issue over CredentialRequests of several request kinds in one call: shape_kinds = list of request kind
+        vectors, requests = uint8 array of the requests concatenated in order (record i is a request of kinds shape_kinds[shape_ids[i]]
+        in the issue_wire layout, 3n + 14 words whatever the kinds), shape_ids = uint8 [count].  Returns (issuances uint8
+        [count][2n + 9][32] in record order, status) -- with the same shape_kinds and shape_ids, what verify_mixed_wire(issuance=True)
+        takes.  out: optional preallocated (e.g. page-locked) contiguous uint8 array of the result's size."""
+        out, status = B.prove_mixed_wire(self._b, self._b.L.afx_issue_mixed_wire, self._h, shape_kinds, requests, shape_ids, True, out)
+        n = len(bytes(shape_kinds[0])) if len(shape_kinds) else 0
+        return out.reshape(len(status), 2 * n + 9, 32), status
+
+    def show_mixed_wire(self, shape_kinds, inputs, shape_ids, out=None):
+        """Batch AnonymousCredential::show over inputs of several disclosure patterns in one call: inputs = uint8 array of the show
+        inputs concatenated in order (record i in the show_wire layout of shape_kinds[shape_ids[i]]).  Returns (the presentations
+        concatenated in record order as one uint8 blob -- with the same shape_kinds and shape_ids, what verify_mixed_wire takes --,
+        status); presentation_offsets gives where each record starts.  out: as for issue_mixed_wire."""
+        return B.prove_mixed_wire(self._b, self._b.L.afx_show_mixed_wire, self._h, shape_kinds, inputs, shape_ids, False, out)
+
+    def presentation_offsets(self, shape_kinds, shape_ids):
+        """Byte offsets [count + 1] of the presentations in a show_mixed_wire blob: record i is blob[offsets[i]:offsets[i + 1]]."""
+        return B.record_offsets(B.mixed_record_bytes(self._b, shape_kinds, "presentation"), shape_ids)
+
     def verify_issuance_batch(self, batch: IssuanceBatch, debug=False):
         """Batch CredentialIssuance::verify (issuer.rs:48-57)."""
         return self._run(self._b.L.afx_verify_issuances, batch, 3, 1, debug)

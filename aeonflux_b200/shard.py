@@ -203,6 +203,13 @@ class MultiGpuIssuer:
         fn = self._b.L.afx_multi_verify_issuances_mixed_wire if issuance else self._b.L.afx_multi_verify_presentations_mixed_wire
         return B.verify_mixed_wire(self._b, fn, self._h, shape_kinds, records, shape_ids, issuance)
 
+    def issue_mixed_wire(self, shape_kinds, requests, shape_ids):
+        """Issuer.issue_mixed_wire across the devices: device k issues records [k*N/G, (k+1)*N/G) -> (issuances, status)."""
+        from . import _binding as B
+        out, status = B.prove_mixed_wire(self._b, self._b.L.afx_multi_issue_mixed_wire, self._h, shape_kinds, requests, shape_ids, True)
+        n = len(bytes(shape_kinds[0])) if len(shape_kinds) else 0
+        return out.reshape(len(status), 2 * n + 9, 32), status
+
     def issue_batch(self, batch):
         """Batch Issuer::issue across the devices (request layout of Issuer.issue_batch) -> (IssuanceBatch, status)."""
         import ctypes

@@ -265,6 +265,36 @@ int afx_show_device(afx_ctx* ctx, uint16_t n_attrs, const uint8_t* kinds, size_t
 int afx_show_wire(afx_ctx* ctx, uint16_t n_attrs, const uint8_t* kinds, size_t count, const uint8_t* inputs, uint8_t* presentations,
                   uint8_t* status);
 
+/* Issue or show over records of SEVERAL shapes of the context's issuer in one call, bucketed on the device: Issuer::issue over
+ * CredentialRequests of several request kinds, or AnonymousCredential::show for users who each chose which attributes to hide.
+ *   shape_kinds = [n_shapes][n_attrs] the kind vectors of the call, 1 <= n_shapes <= 255 (a vector may be listed twice)
+ *   shape_ids   = [count] shape of each record, < n_shapes
+ *   requests / inputs = the input records concatenated in order, record i being one item of its shape as afx_issue_wire /
+ *                 afx_show_wire take it: (3 * n_attrs + 14) * 32 bytes for every request kind vector, or
+ *                 afx_show_num_fields(n_attrs, kinds) * 32 bytes
+ *   issuances / presentations = the output records concatenated in the same order, record i being what the per-shape call writes
+ *                 for it: (2 * n_attrs + 9) * 32 bytes (the attributes echoed), or afx_presentation_num_fields(n_attrs, kinds) * 32
+ *                 bytes.  So the outputs, with the same shape_kinds and shape_ids, are exactly the records argument of
+ *                 afx_verify_issuances_mixed_wire / afx_verify_presentations_mixed_wire.
+ * Output bytes and status[i] are byte-identical to the per-shape *_wire call on record i: status 1 and an all-zero output record for
+ * a malformed input.  Checked before any device work and before anything is written to the outputs or status: AFX_ERR_ARG for
+ * n_shapes out of range, a shape id >= n_shapes, a null pointer with count > 0 (shape_kinds: always) or submissions outstanding;
+ * AFX_ERR_SHAPE for a kind vector that cannot be issued (a request kind other than 0 or 2, or an attribute count other than the
+ * issuer's) or shown; AFX_ERR_NO_SECRET for issuing on a context without the issuer secret (showing needs none).  count = 0 is AFX_OK.
+ * The call works in passes of at most max_batch consecutive records of any mix: the pass's inputs are copied to the device once, as
+ * received; a kernel copies every record into the item-major bucket of its shape; the prover program of each shape present writes
+ * its outputs into a region of its own; a second kernel puts the outputs and status bytes back in record order; one copy each goes
+ * straight into the caller's buffers.  From page-locked memory the copy in of pass i + 1 and the copy out of pass i - 1 run under the
+ * kernels of pass i.  The library keeps no host copy of the inputs, and wipes the device buffers that held them (request rng bytes,
+ * the credential's t, hidden attributes, keypairs) before it returns.  Device memory: the workspace of the largest shape of the call
+ * at max_batch items, plus three [max_batch][largest input record] buffers (the pass as received, twice, and the buckets), two
+ * [max_batch][largest output record] buffers (the outputs in record order, double-buffered), and about
+ * 2 * (6 + (4 * n_shapes + 16) / 256) bytes of bucketing arrays per record of max_batch. */
+int afx_issue_mixed_wire(afx_ctx* ctx, uint16_t n_attrs, const uint8_t* shape_kinds, size_t n_shapes, size_t count,
+                         const uint8_t* requests, const uint8_t* shape_ids, uint8_t* issuances, uint8_t* status);
+int afx_show_mixed_wire(afx_ctx* ctx, uint16_t n_attrs, const uint8_t* shape_kinds, size_t n_shapes, size_t count,
+                        const uint8_t* inputs, const uint8_t* shape_ids, uint8_t* presentations, uint8_t* status);
+
 /* Issue and show in BatchableProof form: zkp 0.7's prove_batchable instead of prove_compact.  The prover is the same (same inputs,
  * blindings, commitments and transcripts, hence the same challenges and responses); only its return value differs: the blinding
  * commitments in place of each challenge.  The outputs are exactly what the BatchableProof verifiers above take:
@@ -380,6 +410,10 @@ int afx_multi_verify_presentations_mixed_wire(afx_multi* m, uint16_t n_attrs, co
 int afx_multi_verify_issuances_mixed_wire(afx_multi* m, uint16_t n_attrs, const uint8_t* shape_kinds, size_t n_shapes, size_t count,
                                           const uint8_t* records, const uint8_t* shape_ids, uint8_t* verdicts);
 int afx_multi_issue(afx_multi* m, const afx_request_batch* batch, const afx_issuance_out* out, uint8_t* status);
+/* afx_issue_mixed_wire across the devices: device k issues records [k*N/G, (k+1)*N/G) and writes that slice of issuances and status
+ * (requests and issuances have one length whatever the request kinds). */
+int afx_multi_issue_mixed_wire(afx_multi* m, uint16_t n_attrs, const uint8_t* shape_kinds, size_t n_shapes, size_t count,
+                               const uint8_t* requests, const uint8_t* shape_ids, uint8_t* issuances, uint8_t* status);
 
 /* Streamed verification of MIXED shapes (BASELINE configs[4]; SURVEY 8d config 5: "bucketed by shape into chunks").  A stream is a
  * sequence of records of several registered shapes, each record the item-major wire bytes of one presentation (issuance = 1: of

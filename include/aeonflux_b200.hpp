@@ -188,6 +188,32 @@ public:
         for (uint8_t s : st) res.push_back(s == 0 ? Result<>::Ok() : Result<>::Err(CredentialError::BadAttribute));
         return {out, res};
     }
+    // ... over CredentialRequests of any of `shape_kinds` in one call: requests = the wire requests concatenated in order (3n + 14
+    // words each), request i of kinds shape_kinds[shape_ids[i]]; bucketed by shape on the device.  Returns the issuances in record
+    // order ([count][2n + 9][32], what the mixed verify_issuances call takes) and a per-item Result.
+    std::pair<std::vector<uint8_t>, std::vector<Result<>>> issue_batch(const std::vector<std::vector<uint8_t>>& shape_kinds, const uint8_t* requests,
+                                                                       const std::vector<uint8_t>& shape_ids) const {
+        const std::vector<uint8_t> flat = flatten_kinds(shape_kinds);
+        const uint16_t n = shape_kinds.empty() ? 0 : (uint16_t)shape_kinds[0].size();
+        std::vector<uint8_t> out(shape_ids.size() * (2 * (size_t)n + 9) * 32), st(shape_ids.size());
+        int rc = afx_issue_mixed_wire(ctx_, n, flat.data(), shape_kinds.size(), shape_ids.size(), requests, shape_ids.data(), out.data(), st.data());
+        if (rc != AFX_OK) throw Error(rc);
+        return {out, status_results(st, CredentialError::BadAttribute)};
+    }
+    // Batch AnonymousCredential::show over inputs of any of `shape_kinds` in one call (each user hides what it chooses): inputs = the
+    // wire show inputs concatenated in order, input i of shape shape_ids[i].  Returns the presentations concatenated in record order
+    // (what the mixed verify_batch takes) and a per-item Result.
+    std::pair<std::vector<uint8_t>, std::vector<Result<>>> show_batch(const std::vector<std::vector<uint8_t>>& shape_kinds, const uint8_t* inputs,
+                                                                      const std::vector<uint8_t>& shape_ids) const {
+        const std::vector<uint8_t> flat = flatten_kinds(shape_kinds);
+        const uint16_t n = shape_kinds.empty() ? 0 : (uint16_t)shape_kinds[0].size();
+        size_t bytes = 0;
+        for (uint8_t s : shape_ids) if (s < shape_kinds.size()) bytes += 32 * afx_presentation_num_fields(n, shape_kinds[s].data());
+        std::vector<uint8_t> out(bytes), st(shape_ids.size());
+        int rc = afx_show_mixed_wire(ctx_, n, flat.data(), shape_kinds.size(), shape_ids.size(), inputs, shape_ids.data(), out.data(), st.data());
+        if (rc != AFX_OK) throw Error(rc);
+        return {out, status_results(st, CredentialError::BadAttribute)};
+    }
     // Batch AnonymousCredential::show (user side; works on a context without the secret key).  batchable: zkp's prove_batchable
     // form, every challenge replaced by that proof's commitments (what verify_batchable takes).
     std::pair<PresentationBatch, std::vector<Result<>>> show_batch(const ShowBatch& s, bool batchable = false) const {
@@ -255,6 +281,15 @@ private:
         std::vector<Result<>> r;
         for (uint8_t x : v) r.push_back(x == 0 ? Result<>::Ok() : Result<>::Err(CredentialError::VerificationFailure));
         return r;
+    }
+    // the kind vectors of a mixed-shape call, concatenated; they all have one attribute count
+    static std::vector<uint8_t> flatten_kinds(const std::vector<std::vector<uint8_t>>& shape_kinds) {
+        std::vector<uint8_t> flat;
+        for (const auto& k : shape_kinds) {
+            if (k.size() != shape_kinds[0].size()) throw std::invalid_argument("every kind vector has the issuer's attribute count");
+            flat.insert(flat.end(), k.begin(), k.end());
+        }
+        return flat;
     }
     std::vector<uint8_t> sp_, ip_, sk_;
     afx_ctx* ctx_ = nullptr;

@@ -149,6 +149,34 @@ impl B200Context {
         Ok(verdicts)
     }
 
+    /// Batch `Issuer::issue` over wire requests of several request kind vectors: `requests` = the requests concatenated in order
+    /// (`3n + 14` words each), request i of kinds `shape_kinds[shape_ids[i]]`.  Returns the issuances in record order (`2n + 9` words
+    /// each, what `verify_mixed_wire(true, ..)` takes) and a status byte per request.
+    pub fn issue_mixed_wire(&self, shape_kinds: &[&[u8]], requests: &[u8], shape_ids: &[u8]) -> Result<(Vec<u8>, Vec<u8>), B200Error> {
+        let (n, flat, out_len) = mixed_prover_shapes(true, shape_kinds, requests, shape_ids)?;
+        let (mut out, mut status) = (vec![0u8; out_len], vec![0u8; shape_ids.len()]);
+        let rc = unsafe {
+            afx_issue_mixed_wire(self.ctx, n, flat.as_ptr(), shape_kinds.len(), shape_ids.len(), requests.as_ptr(), shape_ids.as_ptr(),
+                                 out.as_mut_ptr(), status.as_mut_ptr())
+        };
+        if rc != 0 { return Err(B200Error(rc)); }
+        Ok((out, status))
+    }
+
+    /// Batch `AnonymousCredential::show` over wire show inputs of several disclosure patterns: `inputs` = the inputs concatenated in
+    /// order, input i of shape `shape_kinds[shape_ids[i]]`.  Returns the presentations concatenated in record order (what
+    /// `verify_mixed_wire(false, ..)` takes) and a status byte per input.
+    pub fn show_mixed_wire(&self, shape_kinds: &[&[u8]], inputs: &[u8], shape_ids: &[u8]) -> Result<(Vec<u8>, Vec<u8>), B200Error> {
+        let (n, flat, out_len) = mixed_prover_shapes(false, shape_kinds, inputs, shape_ids)?;
+        let (mut out, mut status) = (vec![0u8; out_len], vec![0u8; shape_ids.len()]);
+        let rc = unsafe {
+            afx_show_mixed_wire(self.ctx, n, flat.as_ptr(), shape_kinds.len(), shape_ids.len(), inputs.as_ptr(), shape_ids.as_ptr(),
+                                out.as_mut_ptr(), status.as_mut_ptr())
+        };
+        if rc != 0 { return Err(B200Error(rc)); }
+        Ok((out, status))
+    }
+
     /// Batch `CredentialIssuance::verify` over struct-of-arrays fields (`attribute[n], t, U, V, challenge, responses[n+5]`).
     pub fn verify_issuances(&self, kinds: &[u8], fields: &[&[u8]]) -> Result<Vec<u8>, B200Error> {
         let n_fields = 2 * kinds.len() + 9;
@@ -213,6 +241,23 @@ fn mixed_shapes(issuance: bool, shape_kinds: &[&[u8]], records: &[u8], shape_ids
     Ok((n as u16, shape_kinds.concat()))
 }
 
+/// The kind vectors of a mixed-shape prover call, flattened, and the length of its output, after checking that `inputs` holds
+/// exactly one input record per shape id (requests for `issue`, show inputs otherwise).
+fn mixed_prover_shapes(issue: bool, shape_kinds: &[&[u8]], inputs: &[u8], shape_ids: &[u8]) -> Result<(u16, Vec<u8>, usize), B200Error> {
+    let n = shape_kinds.first().map_or(0, |k| k.len());
+    if shape_kinds.iter().any(|k| k.len() != n) { return Err(B200Error(-1)); }
+    let sizes: Vec<(usize, usize)> = shape_kinds.iter().map(|k| unsafe {
+        if issue { (32 * (3 * n + 14), 32 * (2 * n + 9)) }
+        else { (32 * afx_show_num_fields(n as u16, k.as_ptr()), 32 * afx_presentation_num_fields(n as u16, k.as_ptr())) }
+    }).collect();
+    let (mut total_in, mut total_out) = (0usize, 0usize);
+    for &s in shape_ids {
+        match sizes.get(s as usize) { Some(&(i, o)) => { total_in += i; total_out += o; } None => return Err(B200Error(-1)) }
+    }
+    if total_in != inputs.len() { return Err(B200Error(-1)); }
+    Ok((n as u16, shape_kinds.concat(), total_out))
+}
+
 /// Several B200s behind one handle (`afx_multi_*`): the library replicates the issuer context on every listed device, keeps one
 /// host thread per device, cuts a batch into contiguous item slices (device k of G takes `[k*N/G, (k+1)*N/G)`) and lets every
 /// device write its slice of the verdict array.  This is what `Issuer::verify_batch` binds when the box has more than one GPU.
@@ -258,6 +303,18 @@ impl B200Multi {
         let rc = unsafe { f(self.m, n, flat.as_ptr(), shape_kinds.len(), shape_ids.len(), records.as_ptr(), shape_ids.as_ptr(), verdicts.as_mut_ptr()) };
         if rc != 0 { return Err(B200Error(rc)); }
         Ok(verdicts)
+    }
+
+    /// `B200Context::issue_mixed_wire` sharded over the devices: device k issues requests `[k*N/G, (k+1)*N/G)`.
+    pub fn issue_mixed_wire(&self, shape_kinds: &[&[u8]], requests: &[u8], shape_ids: &[u8]) -> Result<(Vec<u8>, Vec<u8>), B200Error> {
+        let (n, flat, out_len) = mixed_prover_shapes(true, shape_kinds, requests, shape_ids)?;
+        let (mut out, mut status) = (vec![0u8; out_len], vec![0u8; shape_ids.len()]);
+        let rc = unsafe {
+            afx_multi_issue_mixed_wire(self.m, n, flat.as_ptr(), shape_kinds.len(), shape_ids.len(), requests.as_ptr(), shape_ids.as_ptr(),
+                                       out.as_mut_ptr(), status.as_mut_ptr())
+        };
+        if rc != 0 { return Err(B200Error(rc)); }
+        Ok((out, status))
     }
 
     /// Batch `CredentialIssuance::verify` over item-major wire bytes (`attribute[n], t, U, V, challenge, responses[n+5]` per item).
