@@ -207,24 +207,6 @@ def _as_fields(fields):
     return ptrs, arrs
 
 
-def verify_mixed_wire(binding, fn, handle, shape_kinds, records, shape_ids, issuance):
-    """Marshals afx_[multi_]verify_{presentations,issuances}_mixed_wire: shape_kinds = the kind vectors of the call, records = uint8
-    array holding the records concatenated in order (record i in the wire layout of shape shape_ids[i]), shape_ids = uint8 [count]."""
-    shape_kinds = [bytes(k) for k in shape_kinds]
-    n = len(shape_kinds[0]) if shape_kinds else 0
-    if any(len(k) != n for k in shape_kinds):
-        raise ValueError("every kind vector of a call has the issuer's attribute count")
-    records = np.ascontiguousarray(records, dtype=np.uint8).reshape(-1)
-    ids = np.ascontiguousarray(shape_ids, dtype=np.uint8).reshape(-1)
-    if len(ids) and int(ids.max()) < len(shape_kinds):      # an unknown shape id is the library's error to report
-        sizes = np.array([32 * ((2 * n + 9) if issuance else binding.L.afx_presentation_num_fields(n, k)) for k in shape_kinds], np.int64)
-        if int(sizes[ids].sum()) != records.size:
-            raise ValueError("records must hold exactly one record of its shape per shape id")
-    verdicts = np.zeros(len(ids), np.uint8)
-    binding.check(fn(handle, n, b"".join(shape_kinds), len(shape_kinds), len(ids), records.ctypes.data, ids.ctypes.data, verdicts.ctypes.data))
-    return verdicts
-
-
 def mixed_record_bytes(binding, shape_kinds, what):
     """Record length in bytes of every kind vector of a mixed call: what = "request", "issuance", "show" (a show input) or
     "presentation"."""
@@ -243,29 +225,33 @@ def record_offsets(sizes, shape_ids):
     return offsets
 
 
-def prove_mixed_wire(binding, fn, handle, shape_kinds, inputs, shape_ids, issue, out=None):
-    """Marshals afx_[multi_]{issue,show}_mixed_wire: shape_kinds = the kind vectors of the call, inputs = uint8 array holding the
-    requests (or show inputs) concatenated in order, record i of shape shape_ids[i], shape_ids = uint8 [count].  Returns (the
-    output records concatenated in order as a flat uint8 array, status).  out: optional preallocated (e.g. page-locked) contiguous
-    uint8 array of exactly the output size, returned flattened."""
+def mixed_wire(binding, fn, handle, shape_kinds, records, shape_ids, what, out_what=None, out=None):
+    """Marshals the mixed-shape calls: shape_kinds = the kind vectors of the call, records = uint8 array holding the input records
+    concatenated in order, record i a `what` record (see mixed_record_bytes) of shape shape_ids[i], shape_ids = uint8 [count].
+    afx_[multi_]verify_{presentations,issuances}_mixed_wire (out_what None) return the verdicts.  afx_[multi_]{issue,show}_mixed_wire
+    (out_what "issuance" or "presentation") return (the output records concatenated in order as a flat uint8 array, status); out:
+    optional preallocated (e.g. page-locked) contiguous uint8 array of exactly the output size, returned flattened."""
     shape_kinds = [bytes(k) for k in shape_kinds]
     n = len(shape_kinds[0]) if shape_kinds else 0
     if any(len(k) != n for k in shape_kinds):
         raise ValueError("every kind vector of a call has the issuer's attribute count")
-    inputs = np.ascontiguousarray(inputs, dtype=np.uint8).reshape(-1)
+    records = np.ascontiguousarray(records, dtype=np.uint8).reshape(-1)
     ids = np.ascontiguousarray(shape_ids, dtype=np.uint8).reshape(-1)
     out_bytes = 0
     if len(ids) and int(ids.max()) < len(shape_kinds):      # an unknown shape id is the library's error to report
-        in_sizes = mixed_record_bytes(binding, shape_kinds, "request" if issue else "show")
-        if int(in_sizes[ids].sum()) != inputs.size:
-            raise ValueError("inputs must hold exactly one record of its shape per shape id")
-        out_bytes = int(mixed_record_bytes(binding, shape_kinds, "issuance" if issue else "presentation")[ids].sum())
+        if int(mixed_record_bytes(binding, shape_kinds, what)[ids].sum()) != records.size:
+            raise ValueError("%s must hold exactly one record of its shape per shape id" % ("inputs" if out_what else "records"))
+        if out_what:
+            out_bytes = int(mixed_record_bytes(binding, shape_kinds, out_what)[ids].sum())
+    status = np.zeros(len(ids), np.uint8)
+    args = [handle, n, b"".join(shape_kinds), len(shape_kinds), len(ids), records.ctypes.data, ids.ctypes.data]
+    if not out_what:
+        binding.check(fn(*args, status.ctypes.data))
+        return status
     if out is None:
         out = np.zeros(out_bytes, np.uint8)
     elif out.dtype != np.uint8 or not out.flags.c_contiguous or out.size != out_bytes:
         raise ValueError("out must be a contiguous uint8 array of %d bytes" % out_bytes)
     out = out.reshape(-1)
-    status = np.zeros(len(ids), np.uint8)
-    binding.check(fn(handle, n, b"".join(shape_kinds), len(shape_kinds), len(ids), inputs.ctypes.data, ids.ctypes.data, out.ctypes.data,
-                     status.ctypes.data))
+    binding.check(fn(*args, out.ctypes.data, status.ctypes.data))
     return out, status

@@ -292,10 +292,6 @@ __global__ void __launch_bounds__(BUCKET_TILE) k_bucket_records(BucketArgs a) {
     __syncthreads();
     for (u32 r = t / 32; r < n; r += BUCKET_TILE / 32) bucket_copy(a.records + src[r], a.fields + dst[r], rec_words[ids[r]], t % 32, 32);
 }
-__global__ void __launch_bounds__(256) k_scatter_verdicts(const uint8_t* bucket_verdicts, const u32* slot, uint8_t* verdicts, u32 count) {
-    u32 i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < count) scatter_verdict_job(bucket_verdicts, slot, verdicts, i);
-}
 // Mixed-shape prover calls, the inverse of k_bucket_records: every thread locates one record's output (engine.cuh:unbucket_locate)
 // and scatters its status byte; then each warp copies whole output records back into record order.
 __global__ void __launch_bounds__(BUCKET_TILE) k_unbucket_records(UnbucketArgs a) {
@@ -566,9 +562,6 @@ static void be_launch_verdict(const Workspace& ws, uint8_t* verdicts, be_stream 
     k_verdict<<<grid_for(ws.count, 256, 1), 256, 0, s>>>(ws, verdicts);
 }
 static void be_launch_bucket_records(const BucketArgs& a, be_stream s) { k_bucket_records<<<grid_for(a.count, BUCKET_TILE, 1), BUCKET_TILE, 0, s>>>(a); }
-static void be_launch_scatter_verdicts(const uint8_t* bucket_verdicts, const u32* slot, uint8_t* verdicts, u32 count, be_stream s) {
-    k_scatter_verdicts<<<grid_for(count, 256, 1), 256, 0, s>>>(bucket_verdicts, slot, verdicts, count);
-}
 static void be_launch_unbucket_records(const UnbucketArgs& a, be_stream s) { k_unbucket_records<<<grid_for(a.count, BUCKET_TILE, 1), BUCKET_TILE, 0, s>>>(a); }
 // entries = 2^bits multiples 1..2^bits of every constant point
 static void be_launch_ctab_setup(const u32* d_enc, u32 ncp, u32* d_ctabs, u32* d_encneg, u32* d_bad, int bits, be_stream s) {

@@ -1246,11 +1246,6 @@ AFX_HD void bucket_copy(const u32* src, u32* dst, u32 words, u32 lane, u32 nlane
     for (u32 k = 4 * lane; k < words; k += 4 * nlanes) { load4(q, src + k); store4(dst + k, q); }
 }
 
-// Verdict of record i, read from its bucket's verdict array.
-AFX_HD void scatter_verdict_job(const uint8_t* bucket_verdicts, const u32* slot, uint8_t* verdicts, u32 i) {
-    verdicts[i] = bucket_verdicts[slot[i]];
-}
-
 // ---- mixed-shape prover calls: the inverse of the bucketing, for the prover outputs -------------------------------------------
 // Each shape's prover program writes its output records item-major into its own region (out_base[s]), in bucket order.  Every record
 // goes back to its position in the pass, and its status byte with it.  The rank comes from the slot k_bucket_records wrote; the host

@@ -290,7 +290,7 @@ class Issuer:
         shape shape_ids[i] in the verify_wire layout), shape_ids = uint8 [count].  The records are bucketed by shape on the
         device; verdicts come back in record order."""
         fn = self._b.L.afx_verify_issuances_mixed_wire if issuance else self._b.L.afx_verify_presentations_mixed_wire
-        return B.verify_mixed_wire(self._b, fn, self._h, shape_kinds, records, shape_ids, issuance)
+        return B.mixed_wire(self._b, fn, self._h, shape_kinds, records, shape_ids, "issuance" if issuance else "presentation")
 
     def issue_mixed_wire(self, shape_kinds, requests, shape_ids, out=None):
         """Batch Issuer::issue over CredentialRequests of several request kinds in one call: shape_kinds = list of request kind
@@ -298,7 +298,7 @@ class Issuer:
         in the issue_wire layout, 3n + 14 words whatever the kinds), shape_ids = uint8 [count].  Returns (issuances uint8
         [count][2n + 9][32] in record order, status) -- with the same shape_kinds and shape_ids, what verify_mixed_wire(issuance=True)
         takes.  out: optional preallocated (e.g. page-locked) contiguous uint8 array of the result's size."""
-        out, status = B.prove_mixed_wire(self._b, self._b.L.afx_issue_mixed_wire, self._h, shape_kinds, requests, shape_ids, True, out)
+        out, status = B.mixed_wire(self._b, self._b.L.afx_issue_mixed_wire, self._h, shape_kinds, requests, shape_ids, "request", "issuance", out)
         n = len(bytes(shape_kinds[0])) if len(shape_kinds) else 0
         return out.reshape(len(status), 2 * n + 9, 32), status
 
@@ -307,7 +307,7 @@ class Issuer:
         inputs concatenated in order (record i in the show_wire layout of shape_kinds[shape_ids[i]]).  Returns (the presentations
         concatenated in record order as one uint8 blob -- with the same shape_kinds and shape_ids, what verify_mixed_wire takes --,
         status); presentation_offsets gives where each record starts.  out: as for issue_mixed_wire."""
-        return B.prove_mixed_wire(self._b, self._b.L.afx_show_mixed_wire, self._h, shape_kinds, inputs, shape_ids, False, out)
+        return B.mixed_wire(self._b, self._b.L.afx_show_mixed_wire, self._h, shape_kinds, inputs, shape_ids, "show", "presentation", out)
 
     def presentation_offsets(self, shape_kinds, shape_ids):
         """Byte offsets [count + 1] of the presentations in a show_mixed_wire blob: record i is blob[offsets[i]:offsets[i + 1]]."""

@@ -201,12 +201,12 @@ class MultiGpuIssuer:
         """Issuer.verify_mixed_wire across the devices: device k takes records [k*N/G, (k+1)*N/G) and buckets them itself."""
         from . import _binding as B
         fn = self._b.L.afx_multi_verify_issuances_mixed_wire if issuance else self._b.L.afx_multi_verify_presentations_mixed_wire
-        return B.verify_mixed_wire(self._b, fn, self._h, shape_kinds, records, shape_ids, issuance)
+        return B.mixed_wire(self._b, fn, self._h, shape_kinds, records, shape_ids, "issuance" if issuance else "presentation")
 
     def issue_mixed_wire(self, shape_kinds, requests, shape_ids):
         """Issuer.issue_mixed_wire across the devices: device k issues records [k*N/G, (k+1)*N/G) -> (issuances, status)."""
         from . import _binding as B
-        out, status = B.prove_mixed_wire(self._b, self._b.L.afx_multi_issue_mixed_wire, self._h, shape_kinds, requests, shape_ids, True)
+        out, status = B.mixed_wire(self._b, self._b.L.afx_multi_issue_mixed_wire, self._h, shape_kinds, requests, shape_ids, "request", "issuance")
         n = len(bytes(shape_kinds[0])) if len(shape_kinds) else 0
         return out.reshape(len(status), 2 * n + 9, 32), status
 

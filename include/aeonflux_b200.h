@@ -186,7 +186,7 @@ int afx_verify_issuances_wire(afx_ctx* ctx, uint16_t n_attrs, const uint8_t* kin
  * shape, keeping the record order, the verify program of each shape present runs over its bucket, and the verdicts are put back in
  * record order before one copy to the host.  The host reads only the shape ids.  Device memory: the workspace of the largest shape
  * of the call at max_batch items, plus three [max_batch][largest record] buffers (the pass as received, twice, and the buckets),
- * plus about 2 * (6 + 4 * n_shapes / 256) bytes of bucketing arrays per record of max_batch. */
+ * plus about 2 * (6 + (4 * n_shapes + 16) / 256) bytes of bucketing arrays per record of max_batch. */
 int afx_verify_presentations_mixed_wire(afx_ctx* ctx, uint16_t n_attrs, const uint8_t* shape_kinds, size_t n_shapes, size_t count,
                                         const uint8_t* records, const uint8_t* shape_ids, uint8_t* verdicts);
 int afx_verify_issuances_mixed_wire(afx_ctx* ctx, uint16_t n_attrs, const uint8_t* shape_kinds, size_t n_shapes, size_t count,
@@ -283,11 +283,12 @@ int afx_show_wire(afx_ctx* ctx, uint16_t n_attrs, const uint8_t* kinds, size_t c
  * issuer's) or shown; AFX_ERR_NO_SECRET for issuing on a context without the issuer secret (showing needs none).  count = 0 is AFX_OK.
  * The call works in passes of at most max_batch consecutive records of any mix: the pass's inputs are copied to the device once, as
  * received; a kernel copies every record into the item-major bucket of its shape; the prover program of each shape present writes
- * its outputs into a region of its own; a second kernel puts the outputs and status bytes back in record order; one copy each goes
- * straight into the caller's buffers.  From page-locked memory the copy in of pass i + 1 and the copy out of pass i - 1 run under the
- * kernels of pass i.  The library keeps no host copy of the inputs, and wipes the device buffers that held them (request rng bytes,
- * the credential's t, hidden attributes, keypairs) before it returns.  Device memory: the workspace of the largest shape of the call
- * at max_batch items, plus three [max_batch][largest input record] buffers (the pass as received, twice, and the buckets), two
+ * its outputs into a region of its own; a second kernel puts the outputs and status bytes back in record order.  The outputs go
+ * straight into the caller's buffer in one copy; the status bytes go through the library's page-locked staging, so the status array
+ * need not be page-locked.  With the inputs and outputs in page-locked memory the copy in of pass i + 1 and the copy out of pass
+ * i - 1 run under the kernels of pass i.  The library keeps no host copy of the inputs, and wipes the device buffers that held them
+ * (request rng bytes, the credential's t, hidden attributes, keypairs) before it returns.  Device memory: the workspace of the
+ * largest shape of the call at max_batch items, plus three [max_batch][largest input record] buffers (the pass as received, twice, and the buckets), two
  * [max_batch][largest output record] buffers (the outputs in record order, double-buffered), and about
  * 2 * (6 + (4 * n_shapes + 16) / 256) bytes of bucketing arrays per record of max_batch. */
 int afx_issue_mixed_wire(afx_ctx* ctx, uint16_t n_attrs, const uint8_t* shape_kinds, size_t n_shapes, size_t count,

@@ -155,11 +155,7 @@ public:
     // order, record i of shape shape_ids[i]; bucketed by shape on the device, results in record order
     std::vector<Result<>> verify_batch(const std::vector<std::vector<uint8_t>>& shape_kinds, const uint8_t* records,
                                        const std::vector<uint8_t>& shape_ids) const {
-        std::vector<uint8_t> flat;
-        for (const auto& k : shape_kinds) {
-            if (k.size() != shape_kinds[0].size()) throw std::invalid_argument("every kind vector has the issuer's attribute count");
-            flat.insert(flat.end(), k.begin(), k.end());
-        }
+        const std::vector<uint8_t> flat = flatten_kinds(shape_kinds);
         const uint16_t n = shape_kinds.empty() ? 0 : (uint16_t)shape_kinds[0].size();
         std::vector<uint8_t> v(shape_ids.size());
         int rc = afx_verify_presentations_mixed_wire(ctx_, n, flat.data(), shape_kinds.size(), shape_ids.size(), records, shape_ids.data(), v.data());

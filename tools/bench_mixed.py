@@ -4,7 +4,7 @@
   - records/s of bucketing the same records on the host (a row gather of 32-byte words into one page-locked buffer per shape) plus
     one afx_verify_presentations_wire call per shape, verdicts scattered back to record order;
   - records/s of afx_stream_push + afx_stream_flush with every shape registered on the one context;
-  - the device time of k_bucket_records and k_scatter_verdicts per call (torch.profiler, in a run of its own after the timings);
+  - the device time of k_bucket_records and k_unbucket_records per call (torch.profiler, in a run of its own after the timings);
   - for reference, records/s of one afx_verify_presentations_wire call over as many records of the README-4 shape alone;
   - the GPU's name, power limit and SM clocks, queried in the same run.
 Workloads: `--records` README-4-issuer presentations (distinct, made on the device) in page-locked memory, shuffled at random:
@@ -135,7 +135,7 @@ def main():
     # device time of the bucketing kernels (profiler run after every timing)
     pools, order, pinned, offsets = workload(torch, iss, PATTERNS["mix4"], N, 700)
     result["kernels_mix4"] = kernel_times(torch, lambda: iss.verify_mixed_wire(PATTERNS["mix4"], pinned, order),
-                                          ["k_bucket_records", "k_scatter_verdicts"])
+                                          ["k_bucket_records", "k_unbucket_records"])
     result["gpu_after"] = gpu_info()
     line = json.dumps(result)
     print(line)
